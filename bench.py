@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- polished Mbp/s of the GoldPolish hot path (filter build + 4 ntEdit rounds + guard).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|5] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole workload: for every batch, build the 4 (counting filter,
 filter) pairs from its mapped reads and run the k=32,28,24,20 ntEdit chain over its contigs, then the 0.75 guard.
@@ -322,6 +322,41 @@ def apply_guard(share, out, off, dropped, guard_fn):
     return new_out, new_off, new_dropped, n_rej
 
 
+DUMP_SAMPLE_BASES = 4_000_000     # draft bases of the contigs whose polished bytes are written
+DUMP_MAX_POLISHED = 8_000_000     # polished bytes written at most (32 MB as float32)
+DUMP_FILTER_BATCHES = 3           # batches whose filter payloads are written (3 x 4 x 512 KiB: 25 MB as float32)
+
+
+def dump_outputs(path, share, out, off, dropped, bfs=None):
+    """Write what one pass of the timed path hands its caller, as .npy files of float32/float64 (under 64 MB in all):
+      polished_len, dropped       per contig of the share: length of the polished record, 1 if it was dropped
+      polished_sample             polished bytes of a seeded sample of contigs, concatenated in contig order
+      polished_sample_contigs     the (global) contig indices of that sample
+      filters_sample              [batches, k, BF_BYTES] filter payloads of a seeded sample of batches (when fetched)
+      filters_sample_batches      the (global) batch indices of that sample
+    The samples are drawn from SEED and the input sizes only, so two builds of the project write the same positions."""
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(SEED)
+    out = np.asarray(out)
+    off = np.asarray(off, dtype=np.int64)
+    n = len(share.contigs)
+    order = rng.permutation(n)
+    take = max(1, int(np.searchsorted(np.cumsum(np.diff(share.contig_off)[order]), DUMP_SAMPLE_BASES, side="right")))
+    pick = np.sort(order[:take])
+    sample = np.concatenate([out[off[c]:off[c + 1]] for c in pick] + [np.zeros(0, np.uint8)])[:DUMP_MAX_POLISHED]
+    arrays = {"polished_len": np.diff(off).astype(np.float64), "dropped": np.asarray(dropped).astype(np.float32),
+              "polished_sample": sample.astype(np.float32),
+              "polished_sample_contigs": share.contigs[pick].astype(np.float64)}
+    if bfs is not None:
+        nb = len(share.batches)
+        bsel = np.sort(rng.choice(nb, size=min(DUMP_FILTER_BATCHES, nb), replace=False))
+        arrays["filters_sample"] = np.asarray(bfs)[bsel].astype(np.float32)
+        arrays["filters_sample_batches"] = share.batches[bsel].astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    return arrays
+
+
 def ours(args, rank, world, local_rank):
     import torch
 
@@ -457,12 +492,17 @@ def ours(args, rank, world, local_rank):
     build_kernel_ms_overlapped = st["build_kernel_ms"]  # device timer when overlapped with the edit kernel
     edit_kernel_ms = st["edit_kernel_ms"]
     launches_per_step = allsum(st["build_launches"] + st["polish_launches"])
+    if args.dump_outputs and rank == 0:
+        # the results of the last timed step, before any later pass overwrites them
+        out_d, off_d, dropped_d = ctx.polish_fetch(out=out_h)
+        dump_outputs(args.dump_outputs, sh, out_d, off_d, dropped_d, ctx.build_fetch(out=bf_h) if fetch_filters else None)
+        log(f"[rank {rank}] outputs of the last timed step written to {args.dump_outputs}")
     # roofline leg: the dominant (build) kernel alone, CUDA events on the launching stream around each launch
     # (bounded filter pool: its waves run inside the pipelined pass only -- the kernel's in-step span stands in)
     if fetch_filters:
         ctx.build_run()
         alone = []
-        for _ in range(max(1, min(args.steps, 3))):
+        for _ in range(args.steps):
             ctx.build_run()
             alone.append(ctx.stats()["build_kernel_ms"])
         build_kernel_ms = float(np.mean(alone))
@@ -477,7 +517,7 @@ def ours(args, rank, world, local_rank):
         ctx.build_output(bf_h)
     step_e2e()
     barrier()
-    e2e_steps = max(1, min(args.steps, args.e2e_steps))
+    e2e_steps = args.steps
     t_e2e0 = time.perf_counter()
     for _ in range(e2e_steps):
         gathered = step_e2e()
@@ -647,11 +687,16 @@ def main():
     ap.add_argument("--no-roof", dest="roof", action="store_false")
     ap.add_argument("--ref-bases-per-core", type=float, default=76000.0,
                     help="draft bases per host core in one CPU step (reference arm / cpu_baseline sample)")
-    ap.add_argument("--e2e-steps", type=int, default=5, help="end-to-end steps timed (at most --steps)")
     ap.add_argument("--resident-filters", type=int, default=4096,
                     help="config 5: batches whose filters are resident at once (8 GiB of pool at 4096)")
     ap.add_argument("--separate", action="store_true", help="build, then polish (no overlap of the two kernels)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0's share; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to write")
     w = WORKLOADS[args.config]
     if args.genome_len is not None:
         w["genome_len"] = args.genome_len
