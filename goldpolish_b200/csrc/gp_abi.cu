@@ -441,8 +441,6 @@ int gp_build_stage(gp_ctx* ctx, uint32_t n_batches, const uint64_t* batch_entry_
   if (!ctx || !batch_entry_off || (!entries && n_batches && batch_entry_off[n_batches])) return GP_ERR_ARG;
   cudaSetDevice(ctx->cfg.device);
   const gp_config& c = ctx->cfg;
-  for (uint32_t i = 0; i < c.nk; i++)
-    if (c.k[i] % 4 != 0) GP_FAIL(ctx, GP_ERR_ARG, "building filters needs k values that are multiples of 4");
   const uint64_t n_entries = batch_entry_off[n_batches];
   std::vector<uint64_t> work(n_batches, 0);
   for (uint32_t b = 0; b < n_batches; b++) {
@@ -845,7 +843,7 @@ int gp_debug_nthash(gp_ctx* ctx, uint64_t read_id, uint32_t k, uint64_t* hashes,
 {
   if (!ctx || !hashes || !valid || !n_positions) return GP_ERR_ARG;
   if (read_id >= ctx->n_reads) GP_FAIL(ctx, GP_ERR_ARG, "read_id out of range (upload reads first)");
-  if (k < 4 || k > 32 || k % 4 != 0) GP_FAIL(ctx, GP_ERR_ARG, "k must be a multiple of 4 within 4..32");
+  if (k < 4 || k > 32) GP_FAIL(ctx, GP_ERR_ARG, "k must be within 4..32");
   cudaSetDevice(ctx->cfg.device);
   const uint32_t len = ctx->h_read_len[read_id];
   const uint64_t npos = len >= k ? uint64_t(len) - k + 1 : 0;

@@ -93,7 +93,7 @@ __device__ __forceinline__ void derive_rest(uint64_t h0, const StreamConsts& sc,
 }
 
 // Calls f(step, entry thr, valid, h0, pw) for every step of this warp's runs in rows [row0, row1).
-template<typename F>
+template<bool PARTIAL, typename F>
 __device__ __forceinline__ void for_runs(const LevelParams& p, const LevelCtx& c, const uint64_t* cum, uint32_t batch, uint32_t ki,
                                          const StreamConsts& sc, uint32_t n_steps, uint32_t row0, uint32_t row1, F&& f)
 {
@@ -152,7 +152,7 @@ __device__ __forceinline__ void for_runs(const LevelParams& p, const LevelCtx& c
           m1 = __ldg(p.nm + wbase + rs + 2);
         }
         uint64_t h0 = 0;
-        const bool valid = hash_h0(c.tf, c.tr, cw0, cw1, cm0, cm1, rs * 32u, npos, c.lane, sc, h0);
+        const bool valid = hash_h0<PARTIAL>(c.tf, c.tr, cw0, cw1, cm0, cm1, rs * 32u, npos, c.lane, sc, h0);
         uint32_t pw[4] = { 0xFFFFF0u, 0xFFFFF1u, 0xFFFFF2u, 0xFFFFF3u };
         if (valid) { pw[0] = pack_index(h0); derive_rest(h0, sc, pw); }
         f(s, thr, valid, h0, pw);
@@ -710,19 +710,21 @@ __global__ void __launch_bounds__(kLevelWarps * 32, 3) build_filters_levels_kern
         unsigned long long w_t0 = 0;
         uint32_t w_steps = 0;
         if (threadIdx.x == 0) w_t0 = globaltimer_ns();
-        for_runs(p, c, cum, batch, ki, sc, n_steps, P.row0, P.row1,
-                 [&](uint32_t s, uint32_t thr, bool valid, uint64_t h0, const uint32_t (&pw)[4]) {
-                   const uint32_t t = s * 32u + c.lane;
-                   const bool q = valid && thr > 0u;
-                   if (q) {
+        with_kmer_shape(sc, [&](auto shape) {
+          for_runs<decltype(shape)::value>(p, c, cum, batch, ki, sc, n_steps, P.row0, P.row1,
+                   [&](uint32_t s, uint32_t thr, bool valid, uint64_t h0, const uint32_t (&pw)[4]) {
+                     const uint32_t t = s * 32u + c.lane;
+                     const bool q = valid && thr > 0u;
+                     if (q) {
 #pragma unroll
-                     for (int j = 0; j < 4; j++) red_min(VC + (pw[j] & 0xFFFFFFu), tag | t);
-                     if (thr == 1u) bf_insert(bf, pw);
-                   }
-                   if (valid) ops++;
-                   w_steps++;
-                   surv_append(lst, cnt, q && thr > 1u, h0, t | (thr << kTimeBits), c.lane);
-                 });
+                       for (int j = 0; j < 4; j++) red_min(VC + (pw[j] & 0xFFFFFFu), tag | t);
+                       if (thr == 1u) bf_insert(bf, pw);
+                     }
+                     if (valid) ops++;
+                     w_steps++;
+                     surv_append(lst, cnt, q && thr > 1u, h0, t | (thr << kTimeBits), c.lane);
+                   });
+        });
         if (c.lane == 0) warp_cnt[cb][wib] = cnt;
         if (threadIdx.x == 0 && p.weighted) { cal_ns += globaltimer_ns() - w_t0; cal_steps += w_steps; }
         continue;
@@ -796,20 +798,22 @@ __global__ void __launch_bounds__(kLevelWarps * 32) debug_nthash_kernel(const ui
   const StreamConsts sc = stream_consts(k);
   const uint32_t npos = len - k + 1, lane = threadIdx.x & 31u;
   const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
-  for (uint32_t s = warp; s * 32u < npos; s += nwarps) {
-    const uint64_t w0 = __ldg(pk + wbase + s), w1 = __ldg(pk + wbase + s + 1);
-    const uint32_t m0 = __ldg(nm + wbase + s), m1 = __ldg(nm + wbase + s + 1);
-    uint64_t h0 = 0;
-    const bool ok = hash_h0(tf, tr, w0, w1, m0, m1, s * 32u, npos, lane, sc, h0);
-    const uint32_t pos = s * 32u + lane;
-    if (pos < npos) {
-      valid[pos] = ok ? 1 : 0;
-      uint64_t h1 = h0 * sc.mul1, h2 = h0 * sc.mul2, h3 = h0 * sc.mul3;
-      h1 ^= h1 >> kMultiShift; h2 ^= h2 >> kMultiShift; h3 ^= h3 >> kMultiShift;
-      h[4 * uint64_t(pos) + 0] = ok ? h0 : 0; h[4 * uint64_t(pos) + 1] = ok ? h1 : 0;
-      h[4 * uint64_t(pos) + 2] = ok ? h2 : 0; h[4 * uint64_t(pos) + 3] = ok ? h3 : 0;
+  with_kmer_shape(sc, [&](auto shape) {
+    for (uint32_t s = warp; s * 32u < npos; s += nwarps) {
+      const uint64_t w0 = __ldg(pk + wbase + s), w1 = __ldg(pk + wbase + s + 1);
+      const uint32_t m0 = __ldg(nm + wbase + s), m1 = __ldg(nm + wbase + s + 1);
+      uint64_t h0 = 0;
+      const bool ok = hash_h0<decltype(shape)::value>(tf, tr, w0, w1, m0, m1, s * 32u, npos, lane, sc, h0);
+      const uint32_t pos = s * 32u + lane;
+      if (pos < npos) {
+        valid[pos] = ok ? 1 : 0;
+        uint64_t h1 = h0 * sc.mul1, h2 = h0 * sc.mul2, h3 = h0 * sc.mul3;
+        h1 ^= h1 >> kMultiShift; h2 ^= h2 >> kMultiShift; h3 ^= h3 >> kMultiShift;
+        h[4 * uint64_t(pos) + 0] = ok ? h0 : 0; h[4 * uint64_t(pos) + 1] = ok ? h1 : 0;
+        h[4 * uint64_t(pos) + 2] = ok ? h2 : 0; h[4 * uint64_t(pos) + 3] = ok ? h3 : 0;
+      }
     }
-  }
+  });
 }
 
 void launch_debug_nthash(const uint64_t* pk, const uint32_t* nm, uint64_t wbase, uint32_t len, uint32_t k, uint64_t* h,

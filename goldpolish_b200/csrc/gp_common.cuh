@@ -69,7 +69,7 @@ __host__ __device__ __forceinline__ uint64_t sror1(uint64_t v)
   return ((v >> 1) & 0x7FFFFFFEFFFFFFFFULL) | m;
 }
 // rotate both halves left by s
-__host__ __device__ __forceinline__ uint64_t srol(uint64_t v, uint32_t s)
+__host__ __device__ __forceinline__ constexpr uint64_t srol(uint64_t v, uint32_t s)
 {
   const uint32_t a = s % 31u, b = s % 33u;
   uint64_t hi = v >> 33, lo = v & 0x1FFFFFFFFULL;

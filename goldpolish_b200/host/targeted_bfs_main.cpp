@@ -277,8 +277,8 @@ int main(int argc, char** argv)
   std::vector<unsigned> ks;
   while (a < argc) ks.push_back(unsigned(std::stoi(argv[a++])));
   if (ks.empty() || ks.size() > GP_MAX_K_VALUES) die("need 1..8 k values");
-  for (const unsigned k : ks) // the device hashes 4 packed bases per table lookup and keeps a k-mer in one 64-bit word
-    if (k < 4 || k > 32 || k % 4 != 0) die("k = " + std::to_string(k) + " is not supported: k must be a multiple of 4 within 4..32");
+  for (const unsigned k : ks) // the device keeps a k-mer in one 64-bit word of packed bases
+    if (k < 4 || k > 32) die("k = " + std::to_string(k) + " is not supported: k must be within 4..32");
 
   info("Loading index from " + target_index_path);
   const SeqIndex targets = SeqIndex::load(target_index_path, target_seqs);

@@ -57,7 +57,7 @@ typedef struct {
   uint32_t struct_size;            /* sizeof(gp_config), for ABI growth */
   int32_t device;                  /* CUDA device ordinal */
   uint32_t nk;                     /* number of k values (<= GP_MAX_K_VALUES) */
-  uint32_t k[GP_MAX_K_VALUES];     /* descending, e.g. 32 28 24 20; each 4..32, multiple of 4 for building */
+  uint32_t k[GP_MAX_K_VALUES];     /* descending, e.g. 32 28 24 20; each 4..32 */
   /* ntEdit options, defaults = scripts/goldpolish-ntedit:27 (-d5 -i5 -m1 -X0.5 -Y0.5 -a1) */
   uint32_t max_insertions;         /* -i, 0..5 */
   uint32_t max_deletions;          /* -d, 0..10 */
