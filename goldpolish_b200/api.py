@@ -33,7 +33,7 @@ class _Config(C.Structure):
                 ("max_resident_batches", C.c_uint32), ("use_ratio", C.c_int32),
                 ("missing_threshold", C.c_float), ("edit_threshold", C.c_float), ("keep_counters", C.c_int32),
                 ("prep_mode", C.c_int32), ("prep_k", C.c_uint32), ("to_upper", C.c_int32),
-                ("max_resident_filters", C.c_uint32)]
+                ("max_resident_filters", C.c_uint32), ("track_edits", C.c_int32)]
 
 
 class _Stats(C.Structure):
@@ -47,6 +47,10 @@ class _Stats(C.Structure):
 
 
 READ_ENTRY_DTYPE = np.dtype([("read_id", np.uint32), ("kmer_threshold", np.uint32)])
+EDIT_DTYPE = np.dtype([("pos", np.uint32), ("ref_len", np.uint32), ("alt_len", np.uint32), ("type", np.uint32),
+                       ("allele_off", np.uint64)])  # gp_edit
+EDIT_TYPES = ("SNV", "MNV", "INS", "DEL", "COMPLEX")  # GP_EDIT_SNV .. GP_EDIT_COMPLEX
+EDIT_INSERTED = 0xFFFFFFFF  # GP_EDIT_INSERTED
 
 _lib = None
 
@@ -55,7 +59,8 @@ EXPORTS = ["gp_default_config", "gp_ctx_create", "gp_ctx_destroy", "gp_last_erro
            "gp_build_run", "gp_build_fetch", "gp_build_fetch_cbf", "gp_filters_load", "gp_polish",
            "gp_polish_stage", "gp_polish_run", "gp_polish_fetch", "gp_kmer_threshold", "gp_mappings_cap",
            "gp_guard_rejects", "gp_roof_microbench", "gp_build_round_times", "gp_pipeline_run", "gp_prep", "gp_build_output_host", "gp_host_alloc", "gp_host_free",
-           "gp_build_cta_times", "gp_flagged_bed", "gp_debug_nthash", "gp_reads_begin", "gp_reads_append", "gp_reads_end"]
+           "gp_build_cta_times", "gp_flagged_bed", "gp_debug_nthash", "gp_reads_begin", "gp_reads_append", "gp_reads_end",
+           "gp_polish_fetch_edits"]
 
 
 def load_library():
@@ -112,6 +117,7 @@ def load_library():
     l.gp_host_free.argtypes = [vp]
     l.gp_host_free.restype = None
     l.gp_prep.argtypes = [vp, u32, vp, vp, C.c_int32, u32, C.c_int32, vp, u64, vp]
+    l.gp_polish_fetch_edits.argtypes = [vp, vp, vp, u64, vp, u64, vp]
     _lib = l
     return l
 
@@ -167,7 +173,7 @@ class Context:
 
     def __init__(self, device: int = 0, ks=DEFAULT_KS, max_insertions=5, max_deletions=5, mode=1, mask=1,
                  missing_ratio=0.5, edit_ratio=0.5, jump=3, min_contig_len=100, max_resident_batches=0,
-                 keep_counters=0, prep_mode=0, prep_k=0, to_upper=0, max_resident_filters=0):
+                 keep_counters=0, prep_mode=0, prep_k=0, to_upper=0, max_resident_filters=0, track_edits=False):
         self._l = load_library()
         cfg = _Config()
         self._l.gp_default_config(C.byref(cfg))
@@ -181,6 +187,7 @@ class Context:
         cfg.keep_counters = keep_counters
         cfg.prep_mode, cfg.prep_k, cfg.to_upper = prep_mode, prep_k, to_upper
         cfg.max_resident_filters = max_resident_filters
+        cfg.track_edits = 1 if track_edits else 0
         h = C.c_void_p()
         rc = self._l.gp_ctx_create(C.byref(cfg), C.byref(h))
         if rc != 0:
@@ -311,6 +318,27 @@ class Context:
         self.polish_stage(seqs, offsets, contig_batch)
         self.polish_run()
         return self.polish_fetch(out=out)
+
+    def polish_fetch_edits(self) -> dict:
+        """Edit records of the last polish (needs Context(track_edits=True)), see gp_polish_fetch_edits: a dict of
+        numpy arrays -- "offsets" (n_contigs + 1, records of contig c at [offsets[c], offsets[c + 1])), "pos" (0-based
+        draft position), "ref_len", "alt_len", "type" (index into EDIT_TYPES), "allele_off" and "alleles" (uint8:
+        REF then ALT of record r at alleles[allele_off[r]:])."""
+        off = np.zeros(getattr(self, "_n_contigs", 0) + 1, dtype=np.uint64)
+        need = np.zeros(2, dtype=np.uint64)
+        rc = self._l.gp_polish_fetch_edits(self._h, _ptr(off), None, 0, None, 0, _ptr(need))
+        if rc == -1 and need.any():
+            recs = np.zeros(max(int(need[0]), 1), dtype=EDIT_DTYPE)
+            alleles = np.zeros(max(int(need[1]), 1), dtype=np.uint8)
+            rc = self._l.gp_polish_fetch_edits(self._h, _ptr(off), _ptr(recs), len(recs), _ptr(alleles), alleles.size,
+                                               _ptr(need))
+        else:
+            recs, alleles = np.zeros(0, dtype=EDIT_DTYPE), np.zeros(0, dtype=np.uint8)
+        self._ck(rc)
+        recs, alleles = recs[:int(need[0])], alleles[:int(need[1])]
+        return {"offsets": off, "pos": recs["pos"].copy(), "ref_len": recs["ref_len"].copy(),
+                "alt_len": recs["alt_len"].copy(), "type": recs["type"].copy(), "allele_off": recs["allele_off"].copy(),
+                "alleles": alleles}
 
     # ---- goldpolish-mask / goldpolish-to-upper alone ----
     def prep(self, seqs, offsets, mode: int, k: int = 0, to_upper: int = 0):

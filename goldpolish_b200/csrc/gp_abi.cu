@@ -99,6 +99,14 @@ struct gp_ctx {
   DevBuf d_batch_order, d_batch_done, d_order_pipe;
   DevBuf d_input, d_in_off, d_buf0, d_buf1, d_cap_off, d_cur_len, d_which, d_dropped, d_nodes, d_node_off,
     d_contig_batch, d_order, d_pnext, d_pcounters, d_error, d_out, d_out_off;
+
+  // edit records (cfg.track_edits): origin slices beside d_buf0 / d_buf1, the edit kernel's own result (the optional
+  // mask / to-upper pass moves the records on), and the records derived from them, kept until the next polish
+  bool edits_polish = false;  // the last polish ran with tracking (its records can be derived)
+  bool edits_ready = false;   // ... and they have been
+  uint64_t n_edits = 0, n_allele_bytes = 0;
+  DevBuf d_orig0, d_orig1, d_elen, d_ewhich, d_bnd_off, d_eflags, d_etmp, d_rec_c, d_rec_i, d_rec_j, d_edits, d_alen,
+    d_alleles, d_edit_coff, d_edit_err;
 };
 
 #define GP_FAIL(ctx, code, msg)                                                                              \
@@ -122,13 +130,15 @@ namespace {
 // small device helpers that do not belong to a hot kernel -------------------------------
 __global__ void scatter_contigs_kernel(const char* __restrict__ in, const uint64_t* __restrict__ in_off,
                                        char* __restrict__ buf0, const uint64_t* __restrict__ cap_off,
-                                       uint32_t* __restrict__ cur_len, uint32_t n)
+                                       uint32_t* __restrict__ cur_len, uint32_t* __restrict__ orig0, uint32_t n)
 {
   for (uint32_t c = blockIdx.x; c < n; c += gridDim.x) {
     const uint64_t a = in_off[c];
     const uint32_t len = uint32_t(in_off[c + 1] - a);
     char* dst = buf0 + cap_off[c];
     for (uint32_t i = threadIdx.x; i < len; i += blockDim.x) dst[i] = in[a + i];
+    if (orig0) // edit records: round 0 starts from the identity
+      for (uint32_t i = threadIdx.x; i < len; i += blockDim.x) orig0[cap_off[c] + i] = i;
     if (threadIdx.x == 0) cur_len[c] = len;
   }
 }
@@ -157,6 +167,7 @@ int validate_config(const gp_config& c, std::string& why)
   if (c.prep_mode < 0 || c.prep_mode > 2) { why = "prep_mode must be 0..2"; return GP_ERR_ARG; }
   if (c.prep_mode && (c.prep_k == 0 || c.prep_k > 64)) { why = "prep_k must be within 1..64"; return GP_ERR_ARG; }
   if (!c.use_ratio && (!(c.missing_threshold > 0) || !(c.edit_threshold > 0))) { why = "x / y thresholds must be > 0"; return GP_ERR_ARG; }
+  if (c.track_edits && c.prep_mode == 2) { why = "track_edits cannot be combined with prep_mode 2 (hard-masked bases would read as substitutions)"; return GP_ERR_ARG; }
   return GP_OK;
 }
 
@@ -232,7 +243,10 @@ void gp_ctx_destroy(gp_ctx* ctx)
                      &ctx->d_next, &ctx->d_counters, &ctx->d_step_pre, &ctx->d_batch_max_thr, &ctx->d_V, &ctx->d_alive, &ctx->d_anchor, &ctx->d_entry_rel, &ctx->d_input, &ctx->d_in_off, &ctx->d_buf0, &ctx->d_buf1,
                      &ctx->d_cap_off, &ctx->d_cur_len, &ctx->d_which, &ctx->d_dropped, &ctx->d_nodes, &ctx->d_node_off,
                      &ctx->d_contig_batch, &ctx->d_order, &ctx->d_pnext, &ctx->d_pcounters, &ctx->d_error, &ctx->d_out,
-                     &ctx->d_out_off, &ctx->d_batch_order, &ctx->d_batch_done, &ctx->d_order_pipe, &ctx->d_stream_tab, &ctx->d_cta_times, &ctx->d_bf_slot };
+                     &ctx->d_out_off, &ctx->d_batch_order, &ctx->d_batch_done, &ctx->d_order_pipe, &ctx->d_stream_tab, &ctx->d_cta_times, &ctx->d_bf_slot,
+                     &ctx->d_orig0, &ctx->d_orig1, &ctx->d_elen, &ctx->d_ewhich, &ctx->d_bnd_off, &ctx->d_eflags, &ctx->d_etmp,
+                     &ctx->d_rec_c, &ctx->d_rec_i, &ctx->d_rec_j, &ctx->d_edits, &ctx->d_alen, &ctx->d_alleles, &ctx->d_edit_coff,
+                     &ctx->d_edit_err };
   for (auto* b : bufs) b->release();
   if (ctx->l2_window_set) { cudaCtxResetPersistingL2Cache(); cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0); }
   for (auto& ev : ctx->ev) if (ev) cudaEventDestroy(ev);
@@ -994,6 +1008,10 @@ static int polish_layout(gp_ctx* ctx)
   GP_CUDA(ctx, ctx->d_buf0.ensure(std::max<uint64_t>(ctx->h_cap_off[n], 16)));
   GP_CUDA(ctx, ctx->d_buf1.ensure(std::max<uint64_t>(ctx->h_cap_off[n], 16)));
   GP_CUDA(ctx, ctx->d_nodes.ensure(std::max<uint64_t>(ctx->h_node_off[n], 1) * sizeof(gp::EdNode)));
+  if (ctx->cfg.track_edits) { // origins: 4 B per byte of capacity, same layout
+    GP_CUDA(ctx, ctx->d_orig0.ensure(std::max<uint64_t>(ctx->h_cap_off[n], 16) * 4));
+    GP_CUDA(ctx, ctx->d_orig1.ensure(std::max<uint64_t>(ctx->h_cap_off[n], 16) * 4));
+  }
   GP_CUDA(ctx, ctx->d_cap_off.ensure((size_t(n) + 1) * 8));
   GP_CUDA(ctx, ctx->d_node_off.ensure((size_t(n) + 1) * 8));
   GP_CUDA(ctx, cudaMemcpyAsync(ctx->d_cap_off.p, ctx->h_cap_off.data(), (size_t(n) + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -1044,6 +1062,7 @@ int gp_polish_stage(gp_ctx* ctx, uint32_t n_contigs, const char* seqs, const uin
   if (int rc = polish_layout(ctx)) return rc;
   ctx->polish_staged = true;
   ctx->polish_done = false;
+  ctx->edits_polish = false;
   return GP_OK;
 }
 
@@ -1058,8 +1077,9 @@ static int polish_prepare(gp_ctx* ctx)
   GP_CUDA(ctx, cudaMemsetAsync(ctx->d_error.p, 0, 4, s));
   if (n == 0) return GP_OK;
   const uint32_t grid = std::min<uint32_t>(n, uint32_t(ctx->sm_count) * 8u);
+  uint32_t* orig0 = ctx->cfg.track_edits ? ctx->d_orig0.as<uint32_t>() : nullptr;
   scatter_contigs_kernel<<<grid, 256, 0, s>>>(ctx->d_input.as<char>(), ctx->d_in_off.as<uint64_t>(), ctx->d_buf0.as<char>(),
-                                              ctx->d_cap_off.as<uint64_t>(), ctx->d_cur_len.as<uint32_t>(), n);
+                                              ctx->d_cap_off.as<uint64_t>(), ctx->d_cur_len.as<uint32_t>(), orig0, n);
   GP_CUDA(ctx, cudaGetLastError());
   return GP_OK;
 }
@@ -1111,6 +1131,10 @@ static int polish_edit(gp_ctx* ctx, cudaStream_t es, const uint32_t* order, uint
   }
   p.max_insertions = c.max_insertions; p.max_deletions = c.max_deletions; p.jump = c.jump;
   p.min_contig_len = c.min_contig_len; p.mode = c.mode; p.mask = c.mask;
+  if (c.track_edits) {
+    p.orig[0] = ctx->d_orig0.as<uint32_t>();
+    p.orig[1] = ctx->d_orig1.as<uint32_t>();
+  }
   if (!alongside) GP_CUDA(ctx, cudaEventRecord(ctx->edit_ev[0], es));
   GP_CUDA(ctx, gp::launch_edit(p, ctx->sm_count, es, alongside));
   if (!alongside) GP_CUDA(ctx, cudaEventRecord(ctx->edit_ev[1], es));
@@ -1136,10 +1160,27 @@ static int prep_launch(gp_ctx* ctx, int32_t mode, uint32_t k, int32_t to_upper)
   return GP_OK;
 }
 
+// edit records: the lengths and buffer indices the edit kernel left, before the mask / to-upper pass moves the records on
+// (that pass writes the other buffer, so the kernel's records and origins stay as they are)
+static int keep_edit_result(gp_ctx* ctx)
+{
+  ctx->edits_polish = false;
+  ctx->edits_ready = false;
+  if (!ctx->cfg.track_edits) return GP_OK;
+  const size_t n = std::max<size_t>(ctx->n_contigs, 1);
+  GP_CUDA(ctx, ctx->d_elen.ensure(n * 4));
+  GP_CUDA(ctx, ctx->d_ewhich.ensure(n));
+  GP_CUDA(ctx, cudaMemcpyAsync(ctx->d_elen.p, ctx->d_cur_len.p, n * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+  GP_CUDA(ctx, cudaMemcpyAsync(ctx->d_ewhich.p, ctx->d_which.p, n, cudaMemcpyDeviceToDevice, ctx->stream));
+  ctx->edits_polish = true;
+  return GP_OK;
+}
+
 static int polish_launch(gp_ctx* ctx)
 {
   if (int rc = polish_prepare(ctx)) return rc;
   if (int rc = polish_edit(ctx, ctx->stream, nullptr, 0, nullptr, false)) return rc;
+  if (int rc = keep_edit_result(ctx)) return rc;
   return prep_launch(ctx, ctx->cfg.prep_mode, ctx->cfg.prep_k, ctx->cfg.to_upper);
 }
 
@@ -1196,6 +1237,7 @@ int gp_prep(gp_ctx* ctx, uint32_t n_records, const char* seqs, const uint64_t* o
   if (int rc = prep_launch(ctx, mode, k, to_upper)) return rc;
   ctx->polish_staged = false; // the staged contigs (if any) were replaced
   ctx->polish_done = true;
+  ctx->edits_polish = false;
   return gp_polish_fetch(ctx, out_seqs, out_cap, out_offsets, nullptr);
 }
 
@@ -1311,6 +1353,7 @@ int gp_pipeline_run(gp_ctx* ctx)
     if (int rc = wave_payloads_out(ctx, s, wv, algo == 2 && ctx->bf_host_dev)) return rc;
   }
   ctx->bf_streamed = ctx->bf_host_user && ((algo == 2 && ctx->bf_host_dev) || !ctx->bf_all_resident);
+  if (int rc = keep_edit_result(ctx)) return rc;
   if (int rc = prep_launch(ctx, c.prep_mode, c.prep_k, c.to_upper)) return rc;
   GP_CUDA(ctx, cudaEventRecord(ctx->ev[3], s));
   ctx->pipelined = true;
@@ -1326,15 +1369,14 @@ int gp_pipeline_run(gp_ctx* ctx)
   return GP_OK;
 }
 
-int gp_polish_fetch(gp_ctx* ctx, char* out_seqs, uint64_t out_cap, uint64_t* out_offsets, uint8_t* out_dropped)
+// Lengths and dropped flags of the last polish, once it has run without error: a contig that outgrew its buffers, or
+// the overlapped edit kernel's watchdog, makes the polish run again here
+static int polish_settle(gp_ctx* ctx, std::vector<uint32_t>& len, std::vector<uint8_t>& dropped)
 {
-  if (!ctx || !out_offsets) return GP_ERR_ARG;
-  if (!ctx->polish_done) GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch before gp_polish_run");
-  cudaSetDevice(ctx->cfg.device);
   cudaStream_t s = ctx->stream;
   const uint32_t n = ctx->n_contigs;
-  std::vector<uint32_t> len(n);
-  std::vector<uint8_t> dropped(n);
+  len.resize(n);
+  dropped.resize(n);
   for (;;) {
     int err = 0;
     GP_CUDA(ctx, cudaMemcpyAsync(&err, ctx->d_error.p, 4, cudaMemcpyDeviceToHost, s));
@@ -1359,6 +1401,19 @@ int gp_polish_fetch(gp_ctx* ctx, char* out_seqs, uint64_t out_cap, uint64_t* out
     if (int rc = polish_layout(ctx)) return rc;
     if (int rc = rerun()) return rc;
   }
+  return GP_OK;
+}
+
+int gp_polish_fetch(gp_ctx* ctx, char* out_seqs, uint64_t out_cap, uint64_t* out_offsets, uint8_t* out_dropped)
+{
+  if (!ctx || !out_offsets) return GP_ERR_ARG;
+  if (!ctx->polish_done) GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch before gp_polish_run");
+  cudaSetDevice(ctx->cfg.device);
+  cudaStream_t s = ctx->stream;
+  const uint32_t n = ctx->n_contigs;
+  std::vector<uint32_t> len;
+  std::vector<uint8_t> dropped;
+  if (int rc = polish_settle(ctx, len, dropped)) return rc;
   uint64_t o = 0;
   for (uint32_t i = 0; i < n; i++) {
     out_offsets[i] = o;
@@ -1388,6 +1443,110 @@ int gp_polish(gp_ctx* ctx, uint32_t n_contigs, const char* seqs, const uint64_t*
   if (rc) return rc;
   if ((rc = gp_polish_run(ctx))) return rc;
   return gp_polish_fetch(ctx, out_seqs, out_cap, out_offsets, out_dropped);
+}
+
+// ------------------------------------------------------------------------------------
+// edit records (derived from the polished records and the origin map, gp_edits.cu)
+// ------------------------------------------------------------------------------------
+static int derive_edits(gp_ctx* ctx, const std::vector<uint8_t>& dropped)
+{
+  cudaStream_t s = ctx->stream;
+  const uint32_t n = ctx->n_contigs;
+  std::vector<uint32_t> elen(n);
+  if (n) GP_CUDA(ctx, cudaMemcpyAsync(elen.data(), ctx->d_elen.p, size_t(n) * 4, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  std::vector<uint64_t> bnd(size_t(n) + 1, 0);
+  for (uint32_t c = 0; c < n; c++) bnd[c + 1] = bnd[c] + (dropped[c] ? 0 : uint64_t(elen[c]) + 1);
+  const uint64_t n_bnd = bnd[n];
+  GP_CUDA(ctx, ctx->d_bnd_off.ensure((size_t(n) + 1) * 8));
+  GP_CUDA(ctx, ctx->d_eflags.ensure((n_bnd + 1) * 8));
+  GP_CUDA(ctx, ctx->d_edit_coff.ensure((size_t(n) + 1) * 8));
+  GP_CUDA(ctx, ctx->d_edit_err.ensure(4));
+  GP_CUDA(ctx, cudaMemcpyAsync(ctx->d_bnd_off.p, bnd.data(), (size_t(n) + 1) * 8, cudaMemcpyHostToDevice, s));
+  GP_CUDA(ctx, cudaMemsetAsync(ctx->d_edit_err.p, 0x7F, 4, s)); // atomicMin target
+  gp::EditsInput in;
+  in.n_contigs = n;
+  in.draft = ctx->d_input.as<char>();
+  in.draft_off = ctx->d_in_off.as<uint64_t>();
+  in.buf[0] = ctx->d_buf0.as<char>();
+  in.buf[1] = ctx->d_buf1.as<char>();
+  in.orig[0] = ctx->d_orig0.as<uint32_t>();
+  in.orig[1] = ctx->d_orig1.as<uint32_t>();
+  in.cap_off = ctx->d_cap_off.as<uint64_t>();
+  in.len = ctx->d_elen.as<uint32_t>();
+  in.which = ctx->d_ewhich.as<uint8_t>();
+  in.bnd_off = ctx->d_bnd_off.as<uint64_t>();
+  in.error = ctx->d_edit_err.as<int>();
+  uint64_t* flags = ctx->d_eflags.as<uint64_t>();
+  size_t tmp = 0;
+  GP_CUDA(ctx, gp::edits_count(in, n_bnd, flags, nullptr, tmp, s));
+  GP_CUDA(ctx, ctx->d_etmp.ensure(std::max<size_t>(tmp, 16)));
+  tmp = ctx->d_etmp.cap;
+  GP_CUDA(ctx, gp::edits_count(in, n_bnd, flags, ctx->d_etmp.p, tmp, s));
+  uint64_t total = 0;
+  int bad = 0;
+  GP_CUDA(ctx, cudaMemcpyAsync(&total, flags + n_bnd, 8, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaMemcpyAsync(&bad, ctx->d_edit_err.p, 4, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  if (bad != 0x7F7F7F7F)
+    GP_FAIL(ctx, GP_ERR_STATE, "edit records: the origins of contig " + std::to_string(bad - 1) +
+                               " do not increase strictly along the polished record; no records are derived");
+  const uint32_t n_rec = uint32_t(total);
+  if ((total >> 32) != n_rec) GP_FAIL(ctx, GP_ERR_STATE, "edit records: record starts and ends do not pair up");
+  GP_CUDA(ctx, ctx->d_rec_c.ensure(std::max<size_t>(n_rec, 1) * 4));
+  GP_CUDA(ctx, ctx->d_rec_i.ensure(std::max<size_t>(n_rec, 1) * 4));
+  GP_CUDA(ctx, ctx->d_rec_j.ensure(std::max<size_t>(n_rec, 1) * 4));
+  GP_CUDA(ctx, ctx->d_edits.ensure(std::max<size_t>(n_rec, 1) * sizeof(gp_edit)));
+  GP_CUDA(ctx, ctx->d_alen.ensure((size_t(n_rec) + 1) * 8));
+  tmp = 0;
+  GP_CUDA(ctx, gp::edits_fill(in, n_bnd, flags, n_rec, nullptr, nullptr, nullptr, nullptr, ctx->d_alen.as<uint64_t>(), nullptr,
+                              nullptr, tmp, s));
+  GP_CUDA(ctx, ctx->d_etmp.ensure(std::max<size_t>(tmp, 16)));
+  tmp = ctx->d_etmp.cap;
+  GP_CUDA(ctx, gp::edits_fill(in, n_bnd, flags, n_rec, ctx->d_rec_c.as<uint32_t>(), ctx->d_rec_i.as<uint32_t>(),
+                              ctx->d_rec_j.as<uint32_t>(), ctx->d_edits.as<gp_edit>(), ctx->d_alen.as<uint64_t>(),
+                              ctx->d_edit_coff.as<uint64_t>(), ctx->d_etmp.p, tmp, s));
+  uint64_t bytes = 0;
+  GP_CUDA(ctx, cudaMemcpyAsync(&bytes, ctx->d_alen.as<uint64_t>() + n_rec, 8, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  GP_CUDA(ctx, ctx->d_alleles.ensure(std::max<uint64_t>(bytes, 16)));
+  GP_CUDA(ctx, gp::edits_alleles(in, n_rec, ctx->d_rec_c.as<uint32_t>(), ctx->d_rec_i.as<uint32_t>(), ctx->d_rec_j.as<uint32_t>(),
+                                 ctx->d_alen.as<uint64_t>(), ctx->d_edits.as<gp_edit>(), ctx->d_alleles.as<char>(), s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  ctx->n_edits = n_rec;
+  ctx->n_allele_bytes = bytes;
+  ctx->edits_ready = true;
+  return GP_OK;
+}
+
+int gp_polish_fetch_edits(gp_ctx* ctx, uint64_t* contig_edit_off, gp_edit* edits, uint64_t edits_cap, char* alleles,
+                          uint64_t alleles_cap, uint64_t needed[2])
+{
+  if (!ctx || !contig_edit_off || !needed) return GP_ERR_ARG;
+  if (!ctx->cfg.track_edits) GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch_edits needs gp_config.track_edits = 1");
+  if (!ctx->polish_done || !ctx->edits_polish)
+    GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch_edits before gp_polish_run / gp_pipeline_run");
+  cudaSetDevice(ctx->cfg.device);
+  cudaStream_t s = ctx->stream;
+  std::vector<uint32_t> len;
+  std::vector<uint8_t> dropped;
+  if (int rc = polish_settle(ctx, len, dropped)) return rc;
+  if (!ctx->edits_ready)
+    if (int rc = derive_edits(ctx, dropped)) return rc;
+  const uint32_t n = ctx->n_contigs;
+  needed[0] = ctx->n_edits;
+  needed[1] = ctx->n_allele_bytes;
+  GP_CUDA(ctx, cudaMemcpyAsync(contig_edit_off, ctx->d_edit_coff.p, (size_t(n) + 1) * 8, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  if (edits_cap < ctx->n_edits || alleles_cap < ctx->n_allele_bytes || (ctx->n_edits && !edits) ||
+      (ctx->n_allele_bytes && !alleles))
+    GP_FAIL(ctx, GP_ERR_ARG, "edit record buffers too small (needed[0] records, needed[1] allele bytes)");
+  if (ctx->n_edits)
+    GP_CUDA(ctx, cudaMemcpyAsync(edits, ctx->d_edits.p, ctx->n_edits * sizeof(gp_edit), cudaMemcpyDeviceToHost, s));
+  if (ctx->n_allele_bytes)
+    GP_CUDA(ctx, cudaMemcpyAsync(alleles, ctx->d_alleles.p, ctx->n_allele_bytes, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  return GP_OK;
 }
 
 // ------------------------------------------------------------------------------------

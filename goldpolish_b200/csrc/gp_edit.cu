@@ -1128,8 +1128,12 @@ __device__ __forceinline__ void edit_round(WS& w)
   }
 }
 
-// writeEditsToFile body (:797-935): walk the rope until the first unset node
-__device__ __forceinline__ uint32_t emit_rope(const WS& w, char* dst, uint32_t cap, int& err)
+// writeEditsToFile body (:797-935): walk the rope until the first unset node.  kTrack: every emitted byte also gets its
+// origin -- a draft range's bytes take the origins of the input bytes they copy, an inserted byte GP_EDIT_INSERTED -- so
+// that the map to the original draft is composed over the k chain as the bytes are copied.  A template parameter, not
+// a pointer test: the default instantiation is the kernel without tracking, instruction for instruction.
+template<bool kTrack>
+__device__ __forceinline__ uint32_t emit_rope(const WS& w, char* dst, uint32_t cap, int& err, const uint32_t* oin, uint32_t* oout)
 {
   uint32_t o = 0;
   for (uint32_t i = 0; i < w.nn; i++) {
@@ -1140,11 +1144,17 @@ __device__ __forceinline__ uint32_t emit_rope(const WS& w, char* dst, uint32_t c
       uint32_t cnt = (n.e + 1u >= n.s) ? (n.e + 1u - n.s) : (w.len - n.s);
       if (n.s + cnt > w.len) cnt = w.len - n.s;
       if (o + cnt > cap) { err = 1; return o; }
-      for (uint32_t q = w.lane; q < cnt; q += 32) dst[o + q] = w.seq[n.s + q];
+      for (uint32_t q = w.lane; q < cnt; q += 32) {
+        dst[o + q] = w.seq[n.s + q];
+        if (kTrack) oout[o + q] = oin[n.s + q];
+      }
       o += cnt;
     } else {
       if (o + 1 > cap) { err = 1; return o; }
-      if (w.lane == 0) dst[o] = (char)n.c;
+      if (w.lane == 0) {
+        dst[o] = (char)n.c;
+        if (kTrack) oout[o] = GP_EDIT_INSERTED;
+      }
       o++;
     }
   }
@@ -1157,6 +1167,7 @@ constexpr uint32_t kWarpSmemWords = 2u * (kInsZeroRow + 32u) + 2u * 5u * 32u + 1
 constexpr uint32_t kWarpSmemBytes = kWarpSmemWords * 8u + kVBuf + 32u;                       // + stream ring + re-seed window
 constexpr int kEditSmWarps = 12; // 12 x 32 x 168 registers: the whole register file of an SM
 
+template<bool kTrack>
 __global__ void __launch_bounds__(kEditSmWarps * 32, 1) edit_kernel(EditParams p)
 {
   extern __shared__ __align__(16) uint64_t edit_dyn[];
@@ -1244,7 +1255,8 @@ __global__ void __launch_bounds__(kEditSmWarps * 32, 1) edit_kernel(EditParams p
       edit_round(w);
       __syncwarp();
       int err = w.err;
-      const uint32_t nl = err ? 0u : emit_rope(w, p.buf[cur ^ 1u] + off, cap, err);
+      const uint32_t nl = err ? 0u : emit_rope<kTrack>(w, p.buf[cur ^ 1u] + off, cap, err, kTrack ? p.orig[cur] + off : nullptr,
+                                                       kTrack ? p.orig[cur ^ 1u] + off : nullptr);
       if (err) { if (lane == 0) atomicExch(p.error, 1); break; }
       __syncwarp();
       len = nl;
@@ -1282,20 +1294,23 @@ constexpr int kAlongsideWarps = 3;
 // everything already running, e.g. the build kernel it is meant to run beside)
 void preload_edit()
 {
-  cudaFuncAttributes a;
-  if (cudaFuncGetAttributes(&a, (const void*)edit_kernel) != cudaSuccess) cudaGetLastError();
-  cudaFuncSetAttribute((const void*)edit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kEditSmWarps * int(kWarpSmemBytes));
+  for (const void* f : { (const void*)edit_kernel<false>, (const void*)edit_kernel<true> }) {
+    cudaFuncAttributes a;
+    if (cudaFuncGetAttributes(&a, f) != cudaSuccess) cudaGetLastError();
+    cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, kEditSmWarps * int(kWarpSmemBytes));
+  }
 }
 
 cudaError_t launch_edit(const EditParams& p, int sm_count, cudaStream_t s, int alongside_build)
 {
   if (p.n_contigs == 0) return cudaSuccess;
+  void (*const kern)(EditParams) = p.orig[0] ? edit_kernel<true> : edit_kernel<false>;
   if (alongside_build && std::getenv("GP_EXP_NO_EDIT")) return cudaSuccess; // (experiment: what the build costs in this mode by itself)
   // (function attributes are per device: set on every launch, a cheap host-side call)
-  cudaFuncSetAttribute((const void*)edit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kEditSmWarps * int(kWarpSmemBytes));
+  cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kEditSmWarps * int(kWarpSmemBytes));
   // same shared-memory carve-out as the build kernel (132 KB), so that the two can share an SM; a CTA that owns its
   // SM asks for what it needs
-  cudaFuncSetAttribute((const void*)edit_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, alongside_build == 2 ? 72 : 58);
+  cudaFuncSetAttribute((const void*)kern, cudaFuncAttributePreferredSharedMemoryCarveout, alongside_build == 2 ? 72 : 58);
   if (alongside_build) {
     const uint32_t warps = alongside_build == 2 ? uint32_t(kEditSmWarps) : uint32_t(kAlongsideWarps);
     uint32_t grid = uint32_t(sm_count);
@@ -1311,18 +1326,18 @@ cudaError_t launch_edit(const EditParams& p, int sm_count, cudaStream_t s, int a
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    if (cudaLaunchKernelEx(&cfg, edit_kernel, p) == cudaSuccess) return cudaSuccess;
+    if (cudaLaunchKernelEx(&cfg, kern, p) == cudaSuccess) return cudaSuccess;
     cudaGetLastError(); // no programmatic launch on this driver: an ordinary launch runs after the build (correct, no overlap)
-    edit_kernel<<<grid, warps * 32, warps * kWarpSmemBytes, s>>>(p);
+    kern<<<grid, warps * 32, warps * kWarpSmemBytes, s>>>(p);
     return cudaGetLastError();
   }
   int per_sm = 0;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, edit_kernel, kEditWarps * 32, kEditWarps * kWarpSmemBytes);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kEditWarps * 32, kEditWarps * kWarpSmemBytes);
   if (per_sm < 1) per_sm = 1;
   uint32_t grid = uint32_t(sm_count) * uint32_t(per_sm);
   const uint32_t need = (p.n_contigs + kEditWarps - 1) / kEditWarps;
   if (grid > need) grid = need;
-  edit_kernel<<<grid, kEditWarps * 32, kEditWarps * kWarpSmemBytes, s>>>(p);
+  kern<<<grid, kEditWarps * 32, kEditWarps * kWarpSmemBytes, s>>>(p);
   return cudaGetLastError();
 }
 

@@ -102,7 +102,8 @@ struct EditParams {
   uint32_t insertion_cap[kMaxK];
   uint32_t max_insertions, max_deletions, jump, min_contig_len;
   int32_t mode, mask;
-};
+  uint32_t* orig[2];            // optional (gp_config.track_edits): draft position of every byte of buf[i], 4 B per byte
+};                              // at 4 * cap_off[c]; orig[0] holds the identity before round 0
 
 struct PrepParams {             // goldpolish-mask / goldpolish-to-upper on the resident contigs (gp_prep.cu)
   uint32_t n_contigs;
@@ -131,5 +132,28 @@ void launch_fill_anchor(const uint32_t* step_pre, const uint16_t* entry_rel, uin
 void launch_roof(uint8_t* cbf_pool, uint32_t* bf_pool, uint64_t region, uint32_t iters, uint32_t warps, cudaStream_t s);
 cudaError_t launch_prep(const PrepParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_edit(const EditParams& p, int sm_count, cudaStream_t s, int alongside_build = 0); // 1: sharing SMs with the build kernel, 2: on SMs of its own
+
+// edit records (gp_edits.cu): the polished records against the pristine draft, through the origin map
+struct EditsInput {
+  uint32_t n_contigs;
+  const char* draft;            // pristine drafts, contig c at draft_off[c]
+  const uint64_t* draft_off;    // n_contigs + 1
+  const char* buf[2];           // polished record of contig c: buf[which[c]] + cap_off[c], len[c] bytes
+  const uint32_t* orig[2];      // its origins: orig[which[c]] + cap_off[c]
+  const uint64_t* cap_off;
+  const uint32_t* len;
+  const uint8_t* which;
+  const uint64_t* bnd_off;      // n_contigs + 1: contig c owns the boundaries [bnd_off[c], bnd_off[c+1]) (len + 1, or 0 dropped)
+  int* error;                   // out: 1 + the first contig whose origins do not increase (atomicMin; 0 = none)
+};
+// pass 1: flags[g] = starts | ends << 32 of boundary g (flags[G] = 0), then an exclusive scan of the G + 1 words in place
+cudaError_t edits_count(const EditsInput& in, uint64_t n_bnd, uint64_t* flags, void* tmp, size_t& tmp_bytes, cudaStream_t s);
+// pass 2: records into edits (pos / lengths / type) and their allele bytes into alen (n_rec + 1 words, scanned in place)
+cudaError_t edits_fill(const EditsInput& in, uint64_t n_bnd, const uint64_t* flags, uint32_t n_rec, uint32_t* rec_c,
+                       uint32_t* rec_i, uint32_t* rec_j, gp_edit* edits, uint64_t* alen, uint64_t* contig_edit_off,
+                       void* tmp, size_t& tmp_bytes, cudaStream_t s);
+// pass 3: allele bytes of every record
+cudaError_t edits_alleles(const EditsInput& in, uint32_t n_rec, const uint32_t* rec_c, const uint32_t* rec_i,
+                          const uint32_t* rec_j, const uint64_t* alen, gp_edit* edits, char* alleles, cudaStream_t s);
 
 } // namespace gp

@@ -811,6 +811,56 @@ inline void write_flagged_bed(const std::string& path, const std::vector<std::st
 }
 
 // ---------------------------------------------------------------------------------------
+// edit records (gp_polish_fetch_edits) as VCF 4.2: one ##contig line per input record, records in input order then POS
+// ---------------------------------------------------------------------------------------
+struct EditRecords {
+  std::vector<uint64_t> offsets; // n_contigs + 1
+  std::vector<gp_edit> edits;
+  std::vector<char> alleles;
+};
+
+inline EditRecords fetch_edits(gp_ctx* ctx, uint32_t n_contigs)
+{
+  EditRecords r;
+  r.offsets.assign(size_t(n_contigs) + 1, 0);
+  uint64_t need[2] = { 0, 0 };
+  int rc = gp_polish_fetch_edits(ctx, r.offsets.data(), nullptr, 0, nullptr, 0, need);
+  if (rc == GP_ERR_ARG && (need[0] || need[1])) {
+    r.edits.resize(need[0]);
+    r.alleles.resize(need[1]);
+    rc = gp_polish_fetch_edits(ctx, r.offsets.data(), r.edits.data(), need[0], r.alleles.data(), need[1], need);
+  }
+  check_gp(ctx, rc, "gp_polish_fetch_edits");
+  return r;
+}
+
+// names: CHROM of each input record (its name up to the first whitespace); lengths: draft lengths.  recs == nullptr
+// writes the header only.
+inline void write_edits_vcf(const std::string& path, const std::vector<std::string>& names, const std::vector<uint64_t>& lengths,
+                            const EditRecords* recs)
+{
+  static const char* const kType[] = { "SNV", "MNV", "INS", "DEL", "COMPLEX" };
+  std::ofstream o(path);
+  if (!o.good()) die("cannot write " + path);
+  o << "##fileformat=VCFv4.2\n##source=goldpolish_b200\n";
+  for (size_t c = 0; c < names.size(); c++) o << "##contig=<ID=" << names[c] << ",length=" << lengths[c] << ">\n";
+  o << "##INFO=<ID=TYPE,Number=1,Type=String,Description=\"Edit made by polishing: SNV, MNV, INS, DEL or COMPLEX\">\n";
+  o << "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\n";
+  if (!recs) return;
+  for (size_t c = 0; c < names.size(); c++)
+    for (uint64_t r = recs->offsets[c]; r < recs->offsets[c + 1]; r++) {
+      const gp_edit& e = recs->edits[r];
+      const char* a = recs->alleles.data() + e.allele_off;
+      o << names[c] << '\t' << uint64_t(e.pos) + 1 << "\t.\t";
+      o.write(a, e.ref_len);
+      o << '\t';
+      o.write(a + e.ref_len, e.alt_len);
+      o << "\t.\tPASS\tTYPE=" << (e.type < 5 ? kType[e.type] : "COMPLEX") << '\n';
+    }
+  if (!o.good()) die("cannot write " + path);
+}
+
+// ---------------------------------------------------------------------------------------
 // FASTA/FASTQ reader with kseq semantics: gz or plain, multi-line sequences, name = text up
 // to the first whitespace, comment = rest of the header line
 // ---------------------------------------------------------------------------------------

@@ -2,7 +2,8 @@
 // Same seven positionals (:3-16); the k chain (:20-29) runs inside ONE gp_polish call instead
 // of one ntedit-gr process per k, then the 0.75 size guard (:31-40) picks the result.
 // Only the final chain file is written (named as the script names it); the per-k
-// intermediates of the script are not consumed by anything downstream.
+// intermediates of the script are not consumed by anything downstream.  GP_EDITS_VCF=1 also writes
+// <outfile>.edits.vcf: what the whole chain changed, in draft coordinates (header only when the guard keeps the input).
 #include "gp_host.hpp"
 
 #include <sys/stat.h>
@@ -44,6 +45,8 @@ int main(int argc, char** argv)
     all_payload.insert(all_payload.end(), one.begin(), one.end());
   }
   if (const char* d = std::getenv("GP_DEVICE")) cfg.device = std::atoi(d);
+  const char* vcf_env = std::getenv("GP_EDITS_VCF");
+  cfg.track_edits = vcf_env && std::string(vcf_env) == "1";
   const std::string in_path = base + ".fa";
   struct stat st;
   if (stat(in_path.c_str(), &st) != 0) die("cannot stat " + in_path);
@@ -65,6 +68,8 @@ int main(int argc, char** argv)
     rc = gp_polish_fetch(ctx, out.data(), out.size(), ooff.data(), dropped.data());
   }
   check_gp(ctx, rc, "gp_polish");
+  EditRecords er;
+  if (cfg.track_edits) er = fetch_edits(ctx, uint32_t(recs.size()));
   gp_ctx_destroy(ctx);
   // the chain's last file, named as the script's loop names it (:27-28)
   std::string prev = base;
@@ -95,6 +100,12 @@ int main(int argc, char** argv)
       eoff.push_back(eseq.size());
     }
     write_flagged_bed(bed, names, eseq.data(), eoff);
+  }
+  if (cfg.track_edits) { // the edits of the whole k chain, of what <outfile> will hold: none when the guard keeps the input
+    std::vector<std::string> names;
+    std::vector<uint64_t> lens;
+    for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); lens.push_back(off[i + 1] - off[i]); }
+    write_edits_vcf(outfile + ".edits.vcf", names, lens, gp_guard_rejects(input_size, output_size) ? nullptr : &er);
   }
   if (gp_guard_rejects(input_size, output_size)) { // :31-37
     if (symlink(in_path.c_str(), outfile.c_str()) != 0) die("symlink failed");

@@ -24,6 +24,7 @@ const struct option longopts[] = {                                   // :124-147
   { "verbose", required_argument, nullptr, 'v' }, { "help", no_argument, nullptr, 1 },
   { "version", no_argument, nullptr, 2 },
   { "bed", required_argument, nullptr, 3 }, // extension: write the flagged (soft-masked, -a1) regions as BED rows
+  { "vcf", required_argument, nullptr, 4 }, // extension: write what polishing changed as VCF records (draft coordinates)
   { nullptr, 0, nullptr, 0 }
 };
 void assert_readable(const std::string& p)
@@ -41,7 +42,7 @@ int main(int argc, char** argv)
   gp_default_config(&cfg);
   cfg.max_insertions = 5; cfg.max_deletions = 5; cfg.mode = 0; cfg.mask = 0; // ntedit.cpp:86-87,109,111
   cfg.use_ratio = 0;
-  std::string draft, bloom, bloomrep, prefix, bed;
+  std::string draft, bloom, bloomrep, prefix, bed, vcf;
   unsigned nthreads = 1;
   int snv = 0, verbose = 0;
   bool dieflag = false;
@@ -71,6 +72,7 @@ int main(int argc, char** argv)
     case 1: std::cerr << "ntedit v1.3.5 (goldpolish_b200 GPU drop-in)\n"; return 0;
     case 2: std::cerr << "ntedit version 1.3.5 (goldpolish_b200 GPU drop-in)\n"; return 0;
     case 3: arg >> bed; break;
+    case 4: arg >> vcf; break;
     default: break;
     }
     if (optarg != nullptr && (!arg.eof() || arg.fail())) { // :1944-1947
@@ -109,6 +111,7 @@ int main(int argc, char** argv)
     prefix = o.str();
   }
   if (const char* d = std::getenv("GP_DEVICE")) cfg.device = std::atoi(d);
+  cfg.track_edits = vcf.empty() ? 0 : 1;
 
   const std::vector<FastaRecord> recs = read_fasta(draft);
   std::string all;
@@ -148,6 +151,13 @@ int main(int argc, char** argv)
       eoff.push_back(eseq.size());
     }
     write_flagged_bed(bed, names, eseq.data(), eoff);
+  }
+  if (!vcf.empty()) {
+    const EditRecords er = fetch_edits(ctx, uint32_t(recs.size()));
+    std::vector<std::string> names;
+    std::vector<uint64_t> lens;
+    for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); lens.push_back(off[i + 1] - off[i]); }
+    write_edits_vcf(vcf, names, lens, &er);
   }
   gp_ctx_destroy(ctx);
   return 0;

@@ -23,6 +23,11 @@
  *   gp_guard_rejects     the 0.75 size guard, scripts/goldpolish-ntedit:31-40
  *   gp_flagged_bed       the soft-masked ("flagged") regions of ntEdit -a1, subprojects/ntedit/ntedit.cpp:1131-1146,
  *                        as BED intervals (the reference itself only lower-cases the bases)
+ *   gp_polish_fetch_edits  what polishing changed, per contig, in draft coordinates (VCF-normalised records).  The
+ *                        reference fork writes no such file: its writeEditsToFile pops the substitution records and
+ *                        writes the FASTA only (subprojects/ntedit/ntedit.cpp:797-935; upstream ntEdit's _changes.tsv
+ *                        is gone).  DERIVED from the polished record and a map of each polished base to its draft
+ *                        position, composed over the k chain as the edit kernel copies the bases
  *   gp_kmer_threshold    mappings_bases_to_kmer_threshold, src/goldpolish_targeted_bfs.cpp:45-53
  *   gp_mappings_cap      mappings_num_max, src/goldpolish_targeted_bfs.cpp:96-99
  */
@@ -82,6 +87,9 @@ typedef struct {
    * wave after wave: gp_pipeline_run polishes every wave before its filters go and gp_build_output_host receives the
    * payloads; gp_build_run needs that destination, and a separate gp_polish is not possible. */
   uint32_t max_resident_filters;
+  /* 1: follow every polished base back to the draft position it came from, so that gp_polish_fetch_edits can report
+   * the edits (default 0).  Not combinable with prep_mode 2: hard-masked bases would read as substitutions. */
+  int32_t track_edits;
 } gp_config;
 
 /* one read handed to fill_bfs: index into the uploaded read store + the target's kmer_threshold */
@@ -199,6 +207,32 @@ int gp_prep(gp_ctx* ctx, uint32_t n_records, const char* seqs, const uint64_t* o
  * build kernel, keep_counters) or when the device turned out not to co-schedule the two kernels (the edit kernel's
  * watchdog, checked after the first pass). */
 int gp_pipeline_run(gp_ctx* ctx);
+
+/* ---- edit records ------------------------------------------------------------------- */
+/* With cfg.track_edits the edit kernel maps every polished base to its 0-based position in the ORIGINAL draft contig, or
+ * to GP_EDIT_INSERTED, composing the map over the k chain.  An anchor is a polished base that maps to a draft base
+ * equal to it up to case (soft-masking is not an edit).  Each gap between consecutive anchors (the contig's ends count
+ * as anchors) whose draft span D or polished span O is non-empty is ONE record, normalised as VCF does:
+ *   D and O non-empty: pos = first base of D, ref = D, alt = O (SNV 1/1, MNV n/n, COMPLEX otherwise);
+ *   one of them empty: the left anchor's draft base is prepended to both and pos is that base (INS / DEL); at the
+ *   contig start the right anchor's base is appended instead.
+ * ref and alt are upper-cased.  Changes that cancel over the chain (a base inserted at one k, deleted at the next)
+ * leave no record: the records say what the polished record changed against the draft.  The records describe the
+ * ntEdit chain's output, before the optional goldpolish-mask / to-upper post-pass.  Origins that do not increase along
+ * a contig are an internal error (GP_ERR_STATE), never a silently wrong record. */
+#define GP_EDIT_INSERTED 0xFFFFFFFFu
+#define GP_EDIT_SNV 0u
+#define GP_EDIT_MNV 1u
+#define GP_EDIT_INS 2u
+#define GP_EDIT_DEL 3u
+#define GP_EDIT_COMPLEX 4u
+typedef struct { uint32_t pos, ref_len, alt_len, type; uint64_t allele_off; } gp_edit; /* REF then ALT bytes at alleles[allele_off] */
+/* records of the last gp_polish / gp_pipeline_run, contig order then pos; needs cfg.track_edits.  Like gp_polish_fetch
+ * they come before the 0.75 guard, and a dropped contig has none.
+ * contig_edit_off: n_contigs + 1 (CSR).  Too-small caps -> GP_ERR_ARG with needed[0] = records, needed[1] = allele bytes
+ * (contig_edit_off is filled either way; edits / alleles may be NULL with a cap of 0). */
+int gp_polish_fetch_edits(gp_ctx* ctx, uint64_t* contig_edit_off, gp_edit* edits, uint64_t edits_cap,
+                          char* alleles, uint64_t alleles_cap, uint64_t needed[2]);
 
 /* ---- flagged regions ---------------------------------------------------------------- */
 /* The reference flags what it could not fix by soft-masking: ntEdit -a1 lower-cases the draft base at every position
