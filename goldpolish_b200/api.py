@@ -43,7 +43,7 @@ class _Stats(C.Structure):
                 ("build_kernel_ms", C.c_float), ("edit_kernel_ms", C.c_float),
                 ("build_launches", C.c_uint32), ("polish_launches", C.c_uint32), ("pack_launches", C.c_uint32),
                 ("build_kernel", C.c_uint32), ("build_slots", C.c_uint32), ("polish_reruns", C.c_uint32),
-                ("edit_sms", C.c_uint32)]
+                ("edit_sms", C.c_uint32), ("level_time_bits", C.c_uint32)]
 
 
 READ_ENTRY_DTYPE = np.dtype([("read_id", np.uint32), ("kmer_threshold", np.uint32)])

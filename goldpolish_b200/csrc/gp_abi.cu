@@ -511,6 +511,9 @@ int gp_build_stage(gp_ctx* ctx, uint32_t n_batches, const uint64_t* batch_entry_
     ctx->n_entries = uint32_t(n_entries);
     ctx->alive_words = uint32_t(max_steps + 1);
     ctx->level_time_bits = 16; // occurrence times of the longest stream must fit
+    // GP_LEVEL_TIME_BITS=n (16..26): a higher floor, i.e. narrower epoch tags, so that small inputs reach the tag clears
+    // of the level kernel (the output does not depend on the width)
+    if (const char* f = std::getenv("GP_LEVEL_TIME_BITS")) ctx->level_time_bits = uint32_t(std::min(26, std::max(16, std::atoi(f))));
     while (ctx->level_time_bits < 26 && (max_steps * 32) >> ctx->level_time_bits) ctx->level_time_bits++;
     GP_CUDA(ctx, ctx->d_step_pre.ensure(pre.size() * 4));
     GP_CUDA(ctx, ctx->d_batch_max_thr.ensure(maxthr.size() * 4));
@@ -833,6 +836,7 @@ int gp_build_run(gp_ctx* ctx)
   ctx->stats.build_launches = launches;
   ctx->stats.build_kernel = uint32_t(algo);
   ctx->stats.build_slots = algo == 2 ? ctx->level_slots : 0;
+  ctx->stats.level_time_bits = algo == 2 ? ctx->level_time_bits : 0;
   ctx->filters_ready = ctx->bf_all_resident; // (a later gp_polish needs them all)
   ctx->build_done = true;
   return GP_OK;
@@ -993,12 +997,20 @@ static int polish_layout(gp_ctx* ctx)
 {
   const uint32_t n = ctx->n_contigs;
   const uint32_t g = ctx->grow;
+  // GP_POLISH_CAPS="bytes,nodes" (either may be empty: the default): the first layout gives a contig len + bytes of
+  // buffer and that many rope nodes, so that small inputs reach the overflow re-run of polish_settle
+  int64_t caps[2] = {-1, -1};
+  if (const char* f = std::getenv("GP_POLISH_CAPS")) {
+    const char* comma = std::strchr(f, ',');
+    if (f[0] && f[0] != ',') caps[0] = std::max(0ll, std::atoll(f));
+    if (comma && comma[1]) caps[1] = std::max(1ll, std::atoll(comma + 1)); // (the root node is written unchecked)
+  }
   ctx->h_cap_off.assign(n + 1, 0);
   ctx->h_node_off.assign(n + 1, 0);
   for (uint32_t i = 0; i < n; i++) {
     const uint64_t len = ctx->h_len[i];
-    uint64_t cap = len + (len >> 1) + 4096;
-    uint64_t nodes = (len >> 2) + 2048;
+    uint64_t cap = len + (caps[0] >= 0 ? uint64_t(caps[0]) : (len >> 1) + 4096);
+    uint64_t nodes = caps[1] >= 0 ? uint64_t(caps[1]) : (len >> 2) + 2048;
     cap <<= g; nodes <<= g;
     cap = (cap + 15) & ~15ull;
     if (cap >= (1ull << 32)) { ctx->err = "contig too long for 32-bit positions"; return GP_ERR_ARG; }
@@ -1362,6 +1374,7 @@ int gp_pipeline_run(gp_ctx* ctx)
   ctx->stats.build_launches = launches;
   ctx->stats.build_kernel = uint32_t(algo);
   ctx->stats.build_slots = algo == 2 ? ctx->level_slots : 0;
+  ctx->stats.level_time_bits = algo == 2 ? ctx->level_time_bits : 0;
   ctx->stats.polish_launches = 1 + edit_launches + ((c.prep_mode || c.to_upper) ? 1 : 0);
   ctx->filters_ready = ctx->bf_all_resident;
   ctx->build_done = true;
@@ -1386,10 +1399,9 @@ static int polish_settle(gp_ctx* ctx, std::vector<uint32_t>& len, std::vector<ui
     }
     GP_CUDA(ctx, cudaStreamSynchronize(s));
     if (!err) break;
-    ctx->stats.polish_reruns++;
     // the polish runs again on the device: from the resident filters, or -- when the pool only ever held one wave --
     // as a whole new pass of the pipeline
-    auto rerun = [&]() { return ctx->filters_ready ? polish_launch(ctx) : gp_pipeline_run(ctx); };
+    auto rerun = [&]() { ctx->stats.polish_reruns++; return ctx->filters_ready ? polish_launch(ctx) : gp_pipeline_run(ctx); };
     if (err == 2) { // pipelined edit kernel gave up waiting for filters (no co-residency): plain re-run, filters are final now
       ctx->overlap_state = -1; // remembered here: the re-run below clears d_error before gp_pipeline_run could look at it
       if (int rc = rerun()) return rc;

@@ -120,6 +120,8 @@ typedef struct {
                                (a contig outgrew its buffers, or the overlapped edit kernel's watchdog fired) */
   uint32_t edit_sms;        /* last gp_pipeline_run: SMs the edit kernel had to itself beside the build kernel
                                (0: the two kernels shared every SM, or nothing was overlapped) */
+  uint32_t level_time_bits; /* last build: width of the occurrence times of the level-synchronous kernel (the epoch tags
+                               take the other 32 - level_time_bits bits); 0 when the in-order kernel ran */
 } gp_stats;
 
 void gp_default_config(gp_config* cfg);
