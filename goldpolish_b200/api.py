@@ -33,7 +33,8 @@ class _Config(C.Structure):
                 ("max_resident_batches", C.c_uint32), ("use_ratio", C.c_int32),
                 ("missing_threshold", C.c_float), ("edit_threshold", C.c_float), ("keep_counters", C.c_int32),
                 ("prep_mode", C.c_int32), ("prep_k", C.c_uint32), ("to_upper", C.c_int32),
-                ("max_resident_filters", C.c_uint32), ("track_edits", C.c_int32)]
+                ("max_resident_filters", C.c_uint32), ("track_edits", C.c_int32),
+                ("kmer_support", C.c_int32)]
 
 
 class _Stats(C.Structure):
@@ -60,7 +61,7 @@ EXPORTS = ["gp_default_config", "gp_ctx_create", "gp_ctx_destroy", "gp_last_erro
            "gp_polish_stage", "gp_polish_run", "gp_polish_fetch", "gp_kmer_threshold", "gp_mappings_cap",
            "gp_guard_rejects", "gp_roof_microbench", "gp_build_round_times", "gp_pipeline_run", "gp_prep", "gp_build_output_host", "gp_host_alloc", "gp_host_free",
            "gp_build_cta_times", "gp_flagged_bed", "gp_debug_nthash", "gp_reads_begin", "gp_reads_append", "gp_reads_end",
-           "gp_polish_fetch_edits"]
+           "gp_polish_fetch_edits", "gp_polish_fetch_support"]
 
 
 def load_library():
@@ -118,6 +119,7 @@ def load_library():
     l.gp_host_free.restype = None
     l.gp_prep.argtypes = [vp, u32, vp, vp, C.c_int32, u32, C.c_int32, vp, u64, vp]
     l.gp_polish_fetch_edits.argtypes = [vp, vp, vp, u64, vp, u64, vp]
+    l.gp_polish_fetch_support.argtypes = [vp, vp, vp]
     _lib = l
     return l
 
@@ -173,7 +175,8 @@ class Context:
 
     def __init__(self, device: int = 0, ks=DEFAULT_KS, max_insertions=5, max_deletions=5, mode=1, mask=1,
                  missing_ratio=0.5, edit_ratio=0.5, jump=3, min_contig_len=100, max_resident_batches=0,
-                 keep_counters=0, prep_mode=0, prep_k=0, to_upper=0, max_resident_filters=0, track_edits=False):
+                 keep_counters=0, prep_mode=0, prep_k=0, to_upper=0, max_resident_filters=0, track_edits=False,
+                 kmer_support=False):
         self._l = load_library()
         cfg = _Config()
         self._l.gp_default_config(C.byref(cfg))
@@ -188,6 +191,7 @@ class Context:
         cfg.prep_mode, cfg.prep_k, cfg.to_upper = prep_mode, prep_k, to_upper
         cfg.max_resident_filters = max_resident_filters
         cfg.track_edits = 1 if track_edits else 0
+        cfg.kmer_support = 1 if kmer_support else 0
         h = C.c_void_p()
         rc = self._l.gp_ctx_create(C.byref(cfg), C.byref(h))
         if rc != 0:
@@ -339,6 +343,16 @@ class Context:
         return {"offsets": off, "pos": recs["pos"].copy(), "ref_len": recs["ref_len"].copy(),
                 "alt_len": recs["alt_len"].copy(), "type": recs["type"].copy(), "allele_off": recs["allele_off"].copy(),
                 "alleles": alleles}
+
+    def polish_fetch_support(self):
+        """k-mer support of the last polish (needs Context(kmer_support=True)), see gp_polish_fetch_support:
+        (counts[n_contigs, nk, 4] uint64 -- draft k-mers, draft present, polished k-mers, polished present --,
+        filter_bits_set[n_batches, nk] uint64)."""
+        n = getattr(self, "_n_contigs", 0)
+        counts = np.zeros((max(n, 1), self.nk, 4), dtype=np.uint64)
+        bits = np.zeros((max(self.n_batches, 1), self.nk), dtype=np.uint64)
+        self._ck(self._l.gp_polish_fetch_support(self._h, _ptr(counts), _ptr(bits)))
+        return counts[:n], bits[:self.n_batches]
 
     # ---- goldpolish-mask / goldpolish-to-upper alone ----
     def prep(self, seqs, offsets, mode: int, k: int = 0, to_upper: int = 0):

@@ -107,6 +107,11 @@ struct gp_ctx {
   uint64_t n_edits = 0, n_allele_bytes = 0;
   DevBuf d_orig0, d_orig1, d_elen, d_ewhich, d_bnd_off, d_eflags, d_etmp, d_rec_c, d_rec_i, d_rec_j, d_edits, d_alen,
     d_alleles, d_edit_coff, d_edit_err;
+
+  // k-mer support (cfg.kmer_support): per (contig, k) counts and per (batch, k) set bits, taken in stream order after the
+  // edit kernel of every launch (every wave) while its filters are resident, before the mask / to-upper pass
+  bool support_polish = false; // the last polish counted them
+  DevBuf d_support, d_sup_steps, d_sup_tmp, d_sup_bits;
 };
 
 #define GP_FAIL(ctx, code, msg)                                                                              \
@@ -167,6 +172,7 @@ int validate_config(const gp_config& c, std::string& why)
   if (c.prep_mode < 0 || c.prep_mode > 2) { why = "prep_mode must be 0..2"; return GP_ERR_ARG; }
   if (c.prep_mode && (c.prep_k == 0 || c.prep_k > 64)) { why = "prep_k must be within 1..64"; return GP_ERR_ARG; }
   if (!c.use_ratio && (!(c.missing_threshold > 0) || !(c.edit_threshold > 0))) { why = "x / y thresholds must be > 0"; return GP_ERR_ARG; }
+  if (c.kmer_support < 0 || c.kmer_support > 1) { why = "kmer_support must be 0 or 1"; return GP_ERR_ARG; }
   if (c.track_edits && c.prep_mode == 2) { why = "track_edits cannot be combined with prep_mode 2 (hard-masked bases would read as substitutions)"; return GP_ERR_ARG; }
   return GP_OK;
 }
@@ -188,6 +194,7 @@ void gp_default_config(gp_config* cfg)
   cfg->missing_threshold = 5.0f; cfg->edit_threshold = 9.0f; // ntedit.cpp:88-89
   cfg->jump = 3; cfg->min_contig_len = 100; // ntedit.cpp:94,85
   cfg->max_resident_batches = 0;
+  cfg->track_edits = 0; cfg->kmer_support = 0; // extensions without a reference counterpart: off
 }
 
 const char* gp_last_error(const gp_ctx* ctx) { return ctx ? ctx->err.c_str() : g_create_error.c_str(); }
@@ -246,7 +253,7 @@ void gp_ctx_destroy(gp_ctx* ctx)
                      &ctx->d_out_off, &ctx->d_batch_order, &ctx->d_batch_done, &ctx->d_order_pipe, &ctx->d_stream_tab, &ctx->d_cta_times, &ctx->d_bf_slot,
                      &ctx->d_orig0, &ctx->d_orig1, &ctx->d_elen, &ctx->d_ewhich, &ctx->d_bnd_off, &ctx->d_eflags, &ctx->d_etmp,
                      &ctx->d_rec_c, &ctx->d_rec_i, &ctx->d_rec_j, &ctx->d_edits, &ctx->d_alen, &ctx->d_alleles, &ctx->d_edit_coff,
-                     &ctx->d_edit_err };
+                     &ctx->d_edit_err, &ctx->d_support, &ctx->d_sup_steps, &ctx->d_sup_tmp, &ctx->d_sup_bits };
   for (auto* b : bufs) b->release();
   if (ctx->l2_window_set) { cudaCtxResetPersistingL2Cache(); cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0); }
   for (auto& ev : ctx->ev) if (ev) cudaEventDestroy(ev);
@@ -1075,6 +1082,7 @@ int gp_polish_stage(gp_ctx* ctx, uint32_t n_contigs, const char* seqs, const uin
   ctx->polish_staged = true;
   ctx->polish_done = false;
   ctx->edits_polish = false;
+  ctx->support_polish = false;
   return GP_OK;
 }
 
@@ -1188,10 +1196,66 @@ static int keep_edit_result(gp_ctx* ctx)
   return GP_OK;
 }
 
+// k-mer support: buffers for this polish, counts and bits cleared (stream order: before its first edit kernel)
+static int support_begin(gp_ctx* ctx)
+{
+  ctx->support_polish = false;
+  if (!ctx->cfg.kmer_support) return GP_OK;
+  const uint32_t nk = ctx->cfg.nk;
+  const size_t n = std::max<size_t>(ctx->n_contigs, 1), nb = std::max<size_t>(ctx->n_batches, 1);
+  GP_CUDA(ctx, ctx->d_support.ensure(n * nk * sizeof(gp_kmer_support)));
+  GP_CUDA(ctx, ctx->d_sup_steps.ensure(2 * n * 8));
+  GP_CUDA(ctx, ctx->d_sup_bits.ensure(nb * nk * 8));
+  gp::SupportInput in;
+  std::memset(&in, 0, sizeof in);
+  in.n = ctx->n_contigs;
+  size_t tmp = 0;
+  GP_CUDA(ctx, gp::support_count(in, nullptr, nullptr, tmp, ctx->sm_count, ctx->stream));
+  GP_CUDA(ctx, ctx->d_sup_tmp.ensure(std::max<size_t>(tmp, 16)));
+  GP_CUDA(ctx, cudaMemsetAsync(ctx->d_support.p, 0, n * nk * sizeof(gp_kmer_support), ctx->stream));
+  GP_CUDA(ctx, cudaMemsetAsync(ctx->d_sup_bits.p, 0, nb * nk * 8, ctx->stream));
+  ctx->support_polish = true;
+  return GP_OK;
+}
+
+// k-mer support of the n contigs ids[0 .. n) (nullptr: all) just polished, and the set bits of the batches whose filters
+// are resident for them: batches[0 .. n_batches) (nullptr: 0 .. n_batches - 1)
+static int support_launch(gp_ctx* ctx, const uint32_t* ids, uint32_t n, const uint32_t* batches, uint32_t n_batches)
+{
+  if (!ctx->cfg.kmer_support) return GP_OK;
+  const gp_config& c = ctx->cfg;
+  gp::SupportInput in;
+  std::memset(&in, 0, sizeof in);
+  in.n = n;
+  in.ids = ids;
+  in.draft = ctx->d_input.as<char>();
+  in.draft_off = ctx->d_in_off.as<uint64_t>();
+  in.buf[0] = ctx->d_buf0.as<char>();
+  in.buf[1] = ctx->d_buf1.as<char>();
+  in.cap_off = ctx->d_cap_off.as<uint64_t>();
+  in.len = ctx->d_cur_len.as<uint32_t>();
+  in.which = ctx->d_which.as<uint8_t>();
+  in.dropped = ctx->d_dropped.as<uint8_t>();
+  in.contig_batch = ctx->d_contig_batch.as<uint32_t>();
+  in.bf_pool = ctx->d_bf_pool.as<uint32_t>();
+  in.bf_slot = ctx->bf_all_resident ? nullptr : ctx->d_bf_slot.as<uint32_t>();
+  in.error = ctx->d_error.as<int>();
+  in.counts = ctx->d_support.as<unsigned long long>();
+  in.nk = c.nk;
+  for (uint32_t i = 0; i < c.nk; i++) in.k[i] = c.k[i];
+  size_t tmp = ctx->d_sup_tmp.cap;
+  GP_CUDA(ctx, gp::support_count(in, ctx->d_sup_steps.as<uint64_t>(), ctx->d_sup_tmp.p, tmp, ctx->sm_count, ctx->stream));
+  GP_CUDA(ctx, gp::support_popcount(in.bf_pool, in.bf_slot, batches, 0, n_batches, c.nk, ctx->d_sup_bits.as<unsigned long long>(),
+                                    ctx->stream));
+  return GP_OK;
+}
+
 static int polish_launch(gp_ctx* ctx)
 {
   if (int rc = polish_prepare(ctx)) return rc;
+  if (int rc = support_begin(ctx)) return rc;
   if (int rc = polish_edit(ctx, ctx->stream, nullptr, 0, nullptr, false)) return rc;
+  if (int rc = support_launch(ctx, nullptr, ctx->n_contigs, nullptr, ctx->n_batches)) return rc;
   if (int rc = keep_edit_result(ctx)) return rc;
   return prep_launch(ctx, ctx->cfg.prep_mode, ctx->cfg.prep_k, ctx->cfg.to_upper);
 }
@@ -1250,6 +1314,7 @@ int gp_prep(gp_ctx* ctx, uint32_t n_records, const char* seqs, const uint64_t* o
   ctx->polish_staged = false; // the staged contigs (if any) were replaced
   ctx->polish_done = true;
   ctx->edits_polish = false;
+  ctx->support_polish = false;
   return gp_polish_fetch(ctx, out_seqs, out_cap, out_offsets, nullptr);
 }
 
@@ -1319,6 +1384,7 @@ int gp_pipeline_run(gp_ctx* ctx)
   if (algo == 2)
     if (int rc = build_stream_tab(ctx, s, true)) return rc;
   if (int rc = polish_prepare(ctx)) return rc;
+  if (int rc = support_begin(ctx)) return rc;
   // Per wave: the build kernel signals `launch_dependents` as it starts; the edit kernel (persistent) is launched behind
   // it in the SAME stream with programmatic stream serialization, so it becomes resident while the build runs, takes
   // the wave's contigs in build order and waits for each one's filters.  No event may sit between the two launches;
@@ -1362,6 +1428,9 @@ int gp_pipeline_run(gp_ctx* ctx)
       if (int rc = polish_edit(ctx, s, ctx->d_order_pipe.as<uint32_t>() + c0, c1 - c0, bd, overlap ? (edit_sms ? 2 : 1) : 0)) return rc;
       edit_launches++;
     }
+    // k-mer support of the wave's contigs and filters, before the next wave's pool clear
+    if (int rc = support_launch(ctx, ctx->d_order_pipe.as<uint32_t>() + c0, c1 - c0, ctx->d_batch_order.as<uint32_t>() + ctx->wave_first[wv],
+                                ctx->wave_count[wv])) return rc;
     if (int rc = wave_payloads_out(ctx, s, wv, algo == 2 && ctx->bf_host_dev)) return rc;
   }
   ctx->bf_streamed = ctx->bf_host_user && ((algo == 2 && ctx->bf_host_dev) || !ctx->bf_all_resident);
@@ -1557,6 +1626,27 @@ int gp_polish_fetch_edits(gp_ctx* ctx, uint64_t* contig_edit_off, gp_edit* edits
     GP_CUDA(ctx, cudaMemcpyAsync(edits, ctx->d_edits.p, ctx->n_edits * sizeof(gp_edit), cudaMemcpyDeviceToHost, s));
   if (ctx->n_allele_bytes)
     GP_CUDA(ctx, cudaMemcpyAsync(alleles, ctx->d_alleles.p, ctx->n_allele_bytes, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  return GP_OK;
+}
+
+int gp_polish_fetch_support(gp_ctx* ctx, gp_kmer_support* out, uint64_t* filter_bits_set)
+{
+  if (!ctx) return GP_ERR_ARG;
+  if (!ctx->cfg.kmer_support) GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch_support needs gp_config.kmer_support = 1");
+  if (!ctx->polish_done || !ctx->support_polish)
+    GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch_support before gp_polish_run / gp_pipeline_run");
+  if (!out && ctx->n_contigs) return GP_ERR_ARG;
+  cudaSetDevice(ctx->cfg.device);
+  cudaStream_t s = ctx->stream;
+  std::vector<uint32_t> len;
+  std::vector<uint8_t> dropped;
+  if (int rc = polish_settle(ctx, len, dropped)) return rc;
+  const uint32_t nk = ctx->cfg.nk;
+  if (ctx->n_contigs)
+    GP_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_support.p, size_t(ctx->n_contigs) * nk * sizeof(gp_kmer_support), cudaMemcpyDeviceToHost, s));
+  if (filter_bits_set && ctx->n_batches)
+    GP_CUDA(ctx, cudaMemcpyAsync(filter_bits_set, ctx->d_sup_bits.p, size_t(ctx->n_batches) * nk * 8, cudaMemcpyDeviceToHost, s));
   GP_CUDA(ctx, cudaStreamSynchronize(s));
   return GP_OK;
 }

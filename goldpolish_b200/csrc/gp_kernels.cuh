@@ -156,4 +156,29 @@ cudaError_t edits_fill(const EditsInput& in, uint64_t n_bnd, const uint64_t* fla
 cudaError_t edits_alleles(const EditsInput& in, uint32_t n_rec, const uint32_t* rec_c, const uint32_t* rec_i,
                           const uint32_t* rec_j, const uint64_t* alen, gp_edit* edits, char* alleles, cudaStream_t s);
 
+// k-mer support (gp_support.cu): the draft and the polished record of every contig of a launch against its batch's filters
+struct SupportInput {
+  uint32_t n;                   // contigs of this launch
+  const uint32_t* ids;          // their ids (nullptr: 0 .. n - 1)
+  const char* draft;            // pristine drafts, contig c at draft_off[c]
+  const uint64_t* draft_off;
+  const char* buf[2];           // polished record of contig c: buf[which[c]] + cap_off[c], len[c] bytes (none if dropped[c])
+  const uint64_t* cap_off;
+  const uint32_t* len;
+  const uint8_t* which;
+  const uint8_t* dropped;
+  const uint32_t* contig_batch;
+  const uint32_t* bf_pool;      // (slot * nk + ki) * kBfWords, slot = bf_slot[batch] (the batch itself without a table)
+  const uint32_t* bf_slot;
+  const int* error;             // the polish's error flag: nonzero, nothing is counted (the polish runs again)
+  unsigned long long* counts;   // [contig][k index][draft k-mers, draft present, polished k-mers, polished present], added to
+  uint32_t nk;
+  uint32_t k[kMaxK];
+};
+// steps: 2 n words (record steps, scanned in place); tmp == nullptr: tmp_bytes receives the scan's scratch size
+cudaError_t support_count(const SupportInput& in, uint64_t* steps, void* tmp, size_t& tmp_bytes, int sm_count, cudaStream_t s);
+// set bits of the nk filters of n_batches batches (batches[i], or first_batch + i without a list) into bits[batch * nk + ki]
+cudaError_t support_popcount(const uint32_t* bf_pool, const uint32_t* bf_slot, const uint32_t* batches, uint32_t first_batch,
+                             uint32_t n_batches, uint32_t nk, unsigned long long* bits, cudaStream_t s);
+
 } // namespace gp

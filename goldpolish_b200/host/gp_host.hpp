@@ -861,6 +861,79 @@ inline void write_edits_vcf(const std::string& path, const std::vector<std::stri
 }
 
 // ---------------------------------------------------------------------------------------
+// k-mer support (gp_polish_fetch_support) as a TSV of k-mer completeness and Merqury's QV, per input record and k
+// ---------------------------------------------------------------------------------------
+struct KmerSupport {
+  std::vector<gp_kmer_support> counts; // n_contigs * nk, contig-major
+  std::vector<uint64_t> bits;          // n_batches * nk, batch-major
+};
+
+inline KmerSupport fetch_support(gp_ctx* ctx, uint32_t n_contigs, uint32_t nk, uint32_t n_batches)
+{
+  KmerSupport s;
+  s.counts.resize(std::max<size_t>(size_t(n_contigs) * nk, 1));
+  s.bits.resize(std::max<size_t>(size_t(n_batches) * nk, 1));
+  check_gp(ctx, gp_polish_fetch_support(ctx, s.counts.data(), s.bits.data()), "gp_polish_fetch_support");
+  s.counts.resize(size_t(n_contigs) * nk);
+  s.bits.resize(size_t(n_batches) * nk);
+  return s;
+}
+
+// E = 1 - (1 - missing / kmers)^(1/k), QV = -10 log10(E): "inf" without a missing k-mer, "NA" without a k-mer
+inline std::string kmer_qv(uint64_t kmers, uint64_t missing, uint32_t k)
+{
+  if (kmers == 0) return "NA";
+  if (missing == 0) return "inf";
+  const double e = 1.0 - std::pow(1.0 - double(missing) / double(kmers), 1.0 / double(k));
+  char b[64];
+  std::snprintf(b, sizeof b, "%.4f", -10.0 * std::log10(e) + 0.0); // (+ 0.0: QV 0 prints without a sign)
+  return b;
+}
+
+// names: one per input record, in the order of the counts; polished_is_draft: the 0.75 guard kept the input, so the
+// polished columns describe the draft
+inline void write_kmer_qv(const std::string& path, const std::vector<std::string>& names, const std::vector<uint32_t>& ks,
+                          const KmerSupport& s, bool polished_is_draft)
+{
+  const size_t nk = ks.size(), nb = nk ? s.bits.size() / nk : 0;
+  std::ofstream o(path);
+  if (!o.good()) die("cannot write " + path);
+  char b[64];
+  o << "#goldpolish_b200 k-mer support: k-mers per record position, missing = not contained in the filter of its batch\n#k";
+  for (uint32_t k : ks) o << '\t' << k;
+  o << "\n#filter_fill";
+  for (size_t j = 0; j < nk; j++) { // set bits over all batches' filters of this k
+    uint64_t set = 0;
+    for (size_t bt = 0; bt < nb; bt++) set += s.bits[bt * nk + j];
+    if (nb) std::snprintf(b, sizeof b, "%.6f", double(set) / (double(nb) * 4194304.0));
+    o << '\t' << (nb ? b : "NA");
+  }
+  o << "\n#filter_fp_rate";
+  for (size_t j = 0; j < nk; j++) { // (set / 2^22)^4, the mean over the batches
+    double fp = 0;
+    for (size_t bt = 0; bt < nb; bt++) fp += std::pow(double(s.bits[bt * nk + j]) / 4194304.0, 4.0);
+    if (nb) std::snprintf(b, sizeof b, "%.6g", fp / double(nb));
+    o << '\t' << (nb ? b : "NA");
+  }
+  o << "\n#name\tk\tdraft_kmers\tdraft_missing\tdraft_qv\tpolished_kmers\tpolished_missing\tpolished_qv\n";
+  std::vector<uint64_t> tot(4 * nk, 0);
+  for (size_t c = 0; c < names.size(); c++)
+    for (size_t j = 0; j < nk; j++) {
+      const gp_kmer_support& e = s.counts[c * nk + j];
+      const uint64_t dk = e.draft_kmers, dm = e.draft_kmers - e.draft_present;
+      const uint64_t pk = polished_is_draft ? dk : e.polished_kmers;
+      const uint64_t pm = polished_is_draft ? dm : e.polished_kmers - e.polished_present;
+      o << names[c] << '\t' << ks[j] << '\t' << dk << '\t' << dm << '\t' << kmer_qv(dk, dm, ks[j]) << '\t' << pk << '\t' << pm
+        << '\t' << kmer_qv(pk, pm, ks[j]) << '\n';
+      tot[4 * j] += dk; tot[4 * j + 1] += dm; tot[4 * j + 2] += pk; tot[4 * j + 3] += pm;
+    }
+  for (size_t j = 0; j < nk; j++)
+    o << "*\t" << ks[j] << '\t' << tot[4 * j] << '\t' << tot[4 * j + 1] << '\t' << kmer_qv(tot[4 * j], tot[4 * j + 1], ks[j]) << '\t'
+      << tot[4 * j + 2] << '\t' << tot[4 * j + 3] << '\t' << kmer_qv(tot[4 * j + 2], tot[4 * j + 3], ks[j]) << '\n';
+  if (!o.good()) die("cannot write " + path);
+}
+
+// ---------------------------------------------------------------------------------------
 // FASTA/FASTQ reader with kseq semantics: gz or plain, multi-line sequences, name = text up
 // to the first whitespace, comment = rest of the header line
 // ---------------------------------------------------------------------------------------

@@ -4,6 +4,8 @@
 // Only the final chain file is written (named as the script names it); the per-k
 // intermediates of the script are not consumed by anything downstream.  GP_EDITS_VCF=1 also writes
 // <outfile>.edits.vcf: what the whole chain changed, in draft coordinates (header only when the guard keeps the input).
+// GP_KMER_QV=1 writes <outfile>.kmer_qv.tsv: k-mer completeness and QV of every record, draft and polished, for every k
+// of the chain (when the guard keeps the input, the polished columns describe it).
 #include "gp_host.hpp"
 
 #include <sys/stat.h>
@@ -47,6 +49,8 @@ int main(int argc, char** argv)
   if (const char* d = std::getenv("GP_DEVICE")) cfg.device = std::atoi(d);
   const char* vcf_env = std::getenv("GP_EDITS_VCF");
   cfg.track_edits = vcf_env && std::string(vcf_env) == "1";
+  const char* qv_env = std::getenv("GP_KMER_QV");
+  cfg.kmer_support = qv_env && std::string(qv_env) == "1";
   const std::string in_path = base + ".fa";
   struct stat st;
   if (stat(in_path.c_str(), &st) != 0) die("cannot stat " + in_path);
@@ -70,6 +74,8 @@ int main(int argc, char** argv)
   check_gp(ctx, rc, "gp_polish");
   EditRecords er;
   if (cfg.track_edits) er = fetch_edits(ctx, uint32_t(recs.size()));
+  KmerSupport ks;
+  if (cfg.kmer_support) ks = fetch_support(ctx, uint32_t(recs.size()), cfg.nk, 1);
   gp_ctx_destroy(ctx);
   // the chain's last file, named as the script's loop names it (:27-28)
   std::string prev = base;
@@ -106,6 +112,12 @@ int main(int argc, char** argv)
     std::vector<uint64_t> lens;
     for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); lens.push_back(off[i + 1] - off[i]); }
     write_edits_vcf(outfile + ".edits.vcf", names, lens, gp_guard_rejects(input_size, output_size) ? nullptr : &er);
+  }
+  if (cfg.kmer_support) {
+    std::vector<std::string> names;
+    for (const auto& r : recs) names.push_back(r.name);
+    write_kmer_qv(outfile + ".kmer_qv.tsv", names, std::vector<uint32_t>(cfg.k, cfg.k + cfg.nk), ks,
+                  gp_guard_rejects(input_size, output_size) != 0);
   }
   if (gp_guard_rejects(input_size, output_size)) { // :31-37
     if (symlink(in_path.c_str(), outfile.c_str()) != 0) die("symlink failed");

@@ -25,6 +25,7 @@ const struct option longopts[] = {                                   // :124-147
   { "version", no_argument, nullptr, 2 },
   { "bed", required_argument, nullptr, 3 }, // extension: write the flagged (soft-masked, -a1) regions as BED rows
   { "vcf", required_argument, nullptr, 4 }, // extension: write what polishing changed as VCF records (draft coordinates)
+  { "kmer-qv", required_argument, nullptr, 5 }, // extension: write k-mer completeness / QV of the draft and the polished records
   { nullptr, 0, nullptr, 0 }
 };
 void assert_readable(const std::string& p)
@@ -42,7 +43,7 @@ int main(int argc, char** argv)
   gp_default_config(&cfg);
   cfg.max_insertions = 5; cfg.max_deletions = 5; cfg.mode = 0; cfg.mask = 0; // ntedit.cpp:86-87,109,111
   cfg.use_ratio = 0;
-  std::string draft, bloom, bloomrep, prefix, bed, vcf;
+  std::string draft, bloom, bloomrep, prefix, bed, vcf, kmer_qv;
   unsigned nthreads = 1;
   int snv = 0, verbose = 0;
   bool dieflag = false;
@@ -73,6 +74,7 @@ int main(int argc, char** argv)
     case 2: std::cerr << "ntedit version 1.3.5 (goldpolish_b200 GPU drop-in)\n"; return 0;
     case 3: arg >> bed; break;
     case 4: arg >> vcf; break;
+    case 5: arg >> kmer_qv; break;
     default: break;
     }
     if (optarg != nullptr && (!arg.eof() || arg.fail())) { // :1944-1947
@@ -112,6 +114,7 @@ int main(int argc, char** argv)
   }
   if (const char* d = std::getenv("GP_DEVICE")) cfg.device = std::atoi(d);
   cfg.track_edits = vcf.empty() ? 0 : 1;
+  cfg.kmer_support = kmer_qv.empty() ? 0 : 1;
 
   const std::vector<FastaRecord> recs = read_fasta(draft);
   std::string all;
@@ -158,6 +161,11 @@ int main(int argc, char** argv)
     std::vector<uint64_t> lens;
     for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); lens.push_back(off[i + 1] - off[i]); }
     write_edits_vcf(vcf, names, lens, &er);
+  }
+  if (!kmer_qv.empty()) { // every input record, a dropped one with no polished k-mers
+    std::vector<std::string> names;
+    for (const auto& r : recs) names.push_back(r.name);
+    write_kmer_qv(kmer_qv, names, { cfg.k[0] }, fetch_support(ctx, uint32_t(recs.size()), 1, 1), false);
   }
   gp_ctx_destroy(ctx);
   return 0;

@@ -28,6 +28,9 @@
  *                        writes the FASTA only (subprojects/ntedit/ntedit.cpp:797-935; upstream ntEdit's _changes.tsv
  *                        is gone).  DERIVED from the polished record and a map of each polished base to its draft
  *                        position, composed over the k chain as the edit kernel copies the bases
+ *   gp_polish_fetch_support  k-mer completeness of the draft and of the polished record against the batch's filters,
+ *                        as Merqury reports it from a k-mer database of its own.  No reference counterpart; the counts
+ *                        mirror btllib::NtHash iteration and KmerBloomFilter::contains
  *   gp_kmer_threshold    mappings_bases_to_kmer_threshold, src/goldpolish_targeted_bfs.cpp:45-53
  *   gp_mappings_cap      mappings_num_max, src/goldpolish_targeted_bfs.cpp:96-99
  */
@@ -90,6 +93,9 @@ typedef struct {
   /* 1: follow every polished base back to the draft position it came from, so that gp_polish_fetch_edits can report
    * the edits (default 0).  Not combinable with prep_mode 2: hard-masked bases would read as substitutions. */
   int32_t track_edits;
+  /* 1: count, for every contig and k, how many k-mers of its draft and of its polished record the filters of its batch
+   * contain, so that gp_polish_fetch_support can report k-mer completeness / QV (default 0: no buffers, no launches) */
+  int32_t kmer_support;
 } gp_config;
 
 /* one read handed to fill_bfs: index into the uploaded read store + the target's kmer_threshold */
@@ -235,6 +241,26 @@ typedef struct { uint32_t pos, ref_len, alt_len, type; uint64_t allele_off; } gp
  * (contig_edit_off is filled either way; edits / alleles may be NULL with a cap of 0). */
 int gp_polish_fetch_edits(gp_ctx* ctx, uint64_t* contig_edit_off, gp_edit* edits, uint64_t edits_cap,
                           char* alleles, uint64_t alleles_cap, uint64_t needed[2]);
+
+/* ---- k-mer support ------------------------------------------------------------------ */
+/* With cfg.kmer_support, for contig c and k index j of the chain, against the filter of batch contig_batch[c] for k_j:
+ *   draft_kmers      the k-mers of the DRAFT record that btllib::NtHash iterates (subprojects/ntedit/lib/nthash.hpp roll):
+ *                    one per start position whose k bases are all ACGTacgt; a window holding any other byte (N, IUPAC)
+ *                    is skipped.  Lower-case bases hash as upper-case.  Counted per position, not per distinct k-mer.
+ *   draft_present    how many of those the filter contains, as KmerBloomFilter::contains decides: all 4 bits
+ *                    h_i mod 2^22 set (bit n of a payload is bit n % 8 of byte n / 8)
+ *   polished_kmers / polished_present  the same for the POLISHED record: the ntEdit chain's output before the optional
+ *                    goldpolish-mask / to-upper pass and before the 0.75 guard (the record gp_polish_fetch_edits
+ *                    describes).  0 and 0 for a dropped contig; its draft counts are still reported.
+ * Merqury's QV follows from them on the host: missing = kmers - present, E = 1 - (1 - missing / kmers)^(1/k),
+ * QV = -10 log10(E) (inf when missing = 0, undefined when kmers = 0).  present is biased upward by the filter's false
+ * positive rate (filter_bits_set / 2^22)^4. */
+typedef struct { uint64_t draft_kmers, draft_present, polished_kmers, polished_present; } gp_kmer_support;
+/* counts of the last gp_polish / gp_pipeline_run (on built or gp_filters_load filters); needs cfg.kmer_support, else
+ * GP_ERR_STATE, as before a polish.  out: n_contigs * nk, contig-major.  filter_bits_set (may be NULL): n_batches * nk,
+ * batch-major, the set bits of every filter the polish used.  The same numbers before or after gp_polish_fetch /
+ * gp_polish_fetch_edits (like them it settles a polish that has to run again). */
+int gp_polish_fetch_support(gp_ctx* ctx, gp_kmer_support* out, uint64_t* filter_bits_set);
 
 /* ---- flagged regions ---------------------------------------------------------------- */
 /* The reference flags what it could not fix by soft-masking: ntEdit -a1 lower-cases the draft base at every position
