@@ -50,6 +50,7 @@ class _Stats(C.Structure):
 READ_ENTRY_DTYPE = np.dtype([("read_id", np.uint32), ("kmer_threshold", np.uint32)])
 EDIT_DTYPE = np.dtype([("pos", np.uint32), ("ref_len", np.uint32), ("alt_len", np.uint32), ("type", np.uint32),
                        ("allele_off", np.uint64)])  # gp_edit
+UNSUPPORTED_DTYPE = np.dtype([("start", np.uint32), ("end", np.uint32), ("kmers", np.uint32)])  # gp_unsupported_run
 EDIT_TYPES = ("SNV", "MNV", "INS", "DEL", "COMPLEX")  # GP_EDIT_SNV .. GP_EDIT_COMPLEX
 EDIT_INSERTED = 0xFFFFFFFF  # GP_EDIT_INSERTED
 
@@ -61,7 +62,7 @@ EXPORTS = ["gp_default_config", "gp_ctx_create", "gp_ctx_destroy", "gp_last_erro
            "gp_polish_stage", "gp_polish_run", "gp_polish_fetch", "gp_kmer_threshold", "gp_mappings_cap",
            "gp_guard_rejects", "gp_roof_microbench", "gp_build_round_times", "gp_pipeline_run", "gp_prep", "gp_build_output_host", "gp_host_alloc", "gp_host_free",
            "gp_build_cta_times", "gp_flagged_bed", "gp_debug_nthash", "gp_reads_begin", "gp_reads_append", "gp_reads_end",
-           "gp_polish_fetch_edits", "gp_polish_fetch_support"]
+           "gp_polish_fetch_edits", "gp_polish_fetch_support", "gp_polish_fetch_unsupported"]
 
 
 def load_library():
@@ -120,6 +121,7 @@ def load_library():
     l.gp_prep.argtypes = [vp, u32, vp, vp, C.c_int32, u32, C.c_int32, vp, u64, vp]
     l.gp_polish_fetch_edits.argtypes = [vp, vp, vp, u64, vp, u64, vp]
     l.gp_polish_fetch_support.argtypes = [vp, vp, vp]
+    l.gp_polish_fetch_unsupported.argtypes = [vp, vp, vp, u64, vp]
     _lib = l
     return l
 
@@ -353,6 +355,23 @@ class Context:
         bits = np.zeros((max(self.n_batches, 1), self.nk), dtype=np.uint64)
         self._ck(self._l.gp_polish_fetch_support(self._h, _ptr(counts), _ptr(bits)))
         return counts[:n], bits[:self.n_batches]
+
+    def polish_fetch_unsupported(self) -> dict:
+        """Runs of unsupported k-mers of the last polish (needs Context(kmer_support=True)), see
+        gp_polish_fetch_unsupported: a dict of numpy arrays -- "offsets" (uint64 [n_contigs, 2, nk]: the first run of
+        contig c, record r (0 draft, 1 polished) and k index j), "run_off" (the same n_contigs * 2 * nk + 1 offsets flat:
+        runs of segment i at [run_off[i], run_off[i + 1])), "start", "end" (0-based, half-open) and "kmers" (uint32)."""
+        n = getattr(self, "_n_contigs", 0)
+        off = np.zeros(n * 2 * self.nk + 1, dtype=np.uint64)
+        need = np.zeros(1, dtype=np.uint64)
+        rc = self._l.gp_polish_fetch_unsupported(self._h, _ptr(off), None, 0, _ptr(need))
+        runs = np.zeros(0, dtype=UNSUPPORTED_DTYPE)
+        if rc == -1 and need[0]:
+            runs = np.zeros(int(need[0]), dtype=UNSUPPORTED_DTYPE)
+            rc = self._l.gp_polish_fetch_unsupported(self._h, _ptr(off), _ptr(runs), len(runs), _ptr(need))
+        self._ck(rc)
+        return {"offsets": off[:-1].reshape(n, 2, self.nk), "run_off": off, "start": runs["start"].copy(),
+                "end": runs["end"].copy(), "kmers": runs["kmers"].copy()}
 
     # ---- goldpolish-mask / goldpolish-to-upper alone ----
     def prep(self, seqs, offsets, mode: int, k: int = 0, to_upper: int = 0):

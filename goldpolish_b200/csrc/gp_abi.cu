@@ -112,6 +112,12 @@ struct gp_ctx {
   // edit kernel of every launch (every wave) while its filters are resident, before the mask / to-upper pass
   bool support_polish = false; // the last polish counted them
   DevBuf d_support, d_sup_steps, d_sup_tmp, d_sup_bits;
+  // where the unsupported k-mers lie: the count kernel's bitmap (gp::SupportMiss) and the polished lengths it saw; the
+  // runs derived from them at the first gp_polish_fetch_unsupported
+  uint64_t sup_draft_words = 0, sup_polished_words = 0;
+  bool unsupported_ready = false;
+  uint64_t n_unsupported = 0;
+  DevBuf d_sup_miss, d_sup_len, d_uns_seg, d_uns_runcnt, d_uns_misscnt, d_uns_tmp, d_uns_runs, d_uns_off;
 };
 
 #define GP_FAIL(ctx, code, msg)                                                                              \
@@ -253,7 +259,9 @@ void gp_ctx_destroy(gp_ctx* ctx)
                      &ctx->d_out_off, &ctx->d_batch_order, &ctx->d_batch_done, &ctx->d_order_pipe, &ctx->d_stream_tab, &ctx->d_cta_times, &ctx->d_bf_slot,
                      &ctx->d_orig0, &ctx->d_orig1, &ctx->d_elen, &ctx->d_ewhich, &ctx->d_bnd_off, &ctx->d_eflags, &ctx->d_etmp,
                      &ctx->d_rec_c, &ctx->d_rec_i, &ctx->d_rec_j, &ctx->d_edits, &ctx->d_alen, &ctx->d_alleles, &ctx->d_edit_coff,
-                     &ctx->d_edit_err, &ctx->d_support, &ctx->d_sup_steps, &ctx->d_sup_tmp, &ctx->d_sup_bits };
+                     &ctx->d_edit_err, &ctx->d_support, &ctx->d_sup_steps, &ctx->d_sup_tmp, &ctx->d_sup_bits,
+                     &ctx->d_sup_miss, &ctx->d_sup_len, &ctx->d_uns_seg, &ctx->d_uns_runcnt, &ctx->d_uns_misscnt, &ctx->d_uns_tmp,
+                     &ctx->d_uns_runs, &ctx->d_uns_off };
   for (auto* b : bufs) b->release();
   if (ctx->l2_window_set) { cudaCtxResetPersistingL2Cache(); cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 0); }
   for (auto& ev : ctx->ev) if (ev) cudaEventDestroy(ev);
@@ -1196,21 +1204,29 @@ static int keep_edit_result(gp_ctx* ctx)
   return GP_OK;
 }
 
-// k-mer support: buffers for this polish, counts and bits cleared (stream order: before its first edit kernel)
+// k-mer support: buffers for this polish, counts and bits cleared (stream order: before its first edit kernel).  The
+// bitmap of unsupported starts is sized from the draft lengths and the polished records' capacities of this layout (a
+// re-run after buffer growth comes through here again); it needs no clearing: a record's words are all written by the
+// last count of its contig, and the derivation reads no others.
 static int support_begin(gp_ctx* ctx)
 {
   ctx->support_polish = false;
+  ctx->unsupported_ready = false;
   if (!ctx->cfg.kmer_support) return GP_OK;
   const uint32_t nk = ctx->cfg.nk;
   const size_t n = std::max<size_t>(ctx->n_contigs, 1), nb = std::max<size_t>(ctx->n_batches, 1);
   GP_CUDA(ctx, ctx->d_support.ensure(n * nk * sizeof(gp_kmer_support)));
   GP_CUDA(ctx, ctx->d_sup_steps.ensure(2 * n * 8));
   GP_CUDA(ctx, ctx->d_sup_bits.ensure(nb * nk * 8));
+  ctx->sup_draft_words = ctx->h_in_off[ctx->n_contigs] / 32 + ctx->n_contigs;
+  ctx->sup_polished_words = ctx->h_cap_off[ctx->n_contigs] / 32 + ctx->n_contigs;
+  GP_CUDA(ctx, ctx->d_sup_miss.ensure(std::max<uint64_t>(uint64_t(nk) * (ctx->sup_draft_words + ctx->sup_polished_words), 1) * 4));
+  GP_CUDA(ctx, ctx->d_sup_len.ensure(n * 4));
   gp::SupportInput in;
   std::memset(&in, 0, sizeof in);
   in.n = ctx->n_contigs;
   size_t tmp = 0;
-  GP_CUDA(ctx, gp::support_count(in, nullptr, nullptr, tmp, ctx->sm_count, ctx->stream));
+  GP_CUDA(ctx, gp::support_count(in, gp::SupportMiss{}, nullptr, nullptr, tmp, ctx->sm_count, ctx->stream));
   GP_CUDA(ctx, ctx->d_sup_tmp.ensure(std::max<size_t>(tmp, 16)));
   GP_CUDA(ctx, cudaMemsetAsync(ctx->d_support.p, 0, n * nk * sizeof(gp_kmer_support), ctx->stream));
   GP_CUDA(ctx, cudaMemsetAsync(ctx->d_sup_bits.p, 0, nb * nk * 8, ctx->stream));
@@ -1243,10 +1259,19 @@ static int support_launch(gp_ctx* ctx, const uint32_t* ids, uint32_t n, const ui
   in.counts = ctx->d_support.as<unsigned long long>();
   in.nk = c.nk;
   for (uint32_t i = 0; i < c.nk; i++) in.k[i] = c.k[i];
+  const gp::SupportMiss miss{ ctx->d_sup_miss.as<uint32_t>(), ctx->sup_draft_words, ctx->sup_polished_words };
   size_t tmp = ctx->d_sup_tmp.cap;
-  GP_CUDA(ctx, gp::support_count(in, ctx->d_sup_steps.as<uint64_t>(), ctx->d_sup_tmp.p, tmp, ctx->sm_count, ctx->stream));
+  GP_CUDA(ctx, gp::support_count(in, miss, ctx->d_sup_steps.as<uint64_t>(), ctx->d_sup_tmp.p, tmp, ctx->sm_count, ctx->stream));
   GP_CUDA(ctx, gp::support_popcount(in.bf_pool, in.bf_slot, batches, 0, n_batches, c.nk, ctx->d_sup_bits.as<unsigned long long>(),
                                     ctx->stream));
+  return GP_OK;
+}
+
+// the polished lengths the last counts saw, before the mask / to-upper pass changes them
+static int support_keep(gp_ctx* ctx)
+{
+  if (!ctx->cfg.kmer_support || !ctx->n_contigs) return GP_OK;
+  GP_CUDA(ctx, cudaMemcpyAsync(ctx->d_sup_len.p, ctx->d_cur_len.p, size_t(ctx->n_contigs) * 4, cudaMemcpyDeviceToDevice, ctx->stream));
   return GP_OK;
 }
 
@@ -1256,6 +1281,7 @@ static int polish_launch(gp_ctx* ctx)
   if (int rc = support_begin(ctx)) return rc;
   if (int rc = polish_edit(ctx, ctx->stream, nullptr, 0, nullptr, false)) return rc;
   if (int rc = support_launch(ctx, nullptr, ctx->n_contigs, nullptr, ctx->n_batches)) return rc;
+  if (int rc = support_keep(ctx)) return rc;
   if (int rc = keep_edit_result(ctx)) return rc;
   return prep_launch(ctx, ctx->cfg.prep_mode, ctx->cfg.prep_k, ctx->cfg.to_upper);
 }
@@ -1434,6 +1460,7 @@ int gp_pipeline_run(gp_ctx* ctx)
     if (int rc = wave_payloads_out(ctx, s, wv, algo == 2 && ctx->bf_host_dev)) return rc;
   }
   ctx->bf_streamed = ctx->bf_host_user && ((algo == 2 && ctx->bf_host_dev) || !ctx->bf_all_resident);
+  if (int rc = support_keep(ctx)) return rc;
   if (int rc = keep_edit_result(ctx)) return rc;
   if (int rc = prep_launch(ctx, c.prep_mode, c.prep_k, c.to_upper)) return rc;
   GP_CUDA(ctx, cudaEventRecord(ctx->ev[3], s));
@@ -1648,6 +1675,88 @@ int gp_polish_fetch_support(gp_ctx* ctx, gp_kmer_support* out, uint64_t* filter_
   if (filter_bits_set && ctx->n_batches)
     GP_CUDA(ctx, cudaMemcpyAsync(filter_bits_set, ctx->d_sup_bits.p, size_t(ctx->n_batches) * nk * 8, cudaMemcpyDeviceToHost, s));
   GP_CUDA(ctx, cudaStreamSynchronize(s));
+  return GP_OK;
+}
+
+// runs of unsupported k-mers (gp_support.cu): segments (contig, record, k) of the bitmap as one flat range of words,
+// counted, scanned and filled on the device
+static int derive_unsupported(gp_ctx* ctx, const std::vector<uint8_t>& dropped)
+{
+  cudaStream_t s = ctx->stream;
+  const uint32_t n = ctx->n_contigs, nk = ctx->cfg.nk, n_seg = n * 2 * nk;
+  std::vector<uint32_t> plen(n);
+  if (n) GP_CUDA(ctx, cudaMemcpyAsync(plen.data(), ctx->d_sup_len.p, size_t(n) * 4, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  std::vector<uint64_t> seg(size_t(n_seg) + 1, 0);
+  for (uint32_t c = 0; c < n; c++)
+    for (uint32_t r = 0; r < 2; r++) {
+      // lengths as support_count_kernel reads the records
+      const uint64_t len = r ? (dropped[c] ? 0 : std::min<uint64_t>(plen[c], ctx->h_cap_off[c + 1] - ctx->h_cap_off[c]))
+                             : ctx->h_in_off[c + 1] - ctx->h_in_off[c];
+      for (uint32_t j = 0; j < nk; j++) {
+        const size_t i = (size_t(c) * 2 + r) * nk + j;
+        seg[i + 1] = seg[i] + (len >= ctx->cfg.k[j] ? (len + 31) / 32 : 0);
+      }
+    }
+  const uint64_t n_words = seg[n_seg];
+  GP_CUDA(ctx, ctx->d_uns_seg.ensure((size_t(n_seg) + 1) * 8));
+  GP_CUDA(ctx, ctx->d_uns_off.ensure((size_t(n_seg) + 1) * 8));
+  GP_CUDA(ctx, ctx->d_uns_runcnt.ensure(std::max<uint64_t>(n_words, 1) * 8));
+  GP_CUDA(ctx, ctx->d_uns_misscnt.ensure(std::max<uint64_t>(n_words, 1) * 4));
+  GP_CUDA(ctx, cudaMemcpyAsync(ctx->d_uns_seg.p, seg.data(), (size_t(n_seg) + 1) * 8, cudaMemcpyHostToDevice, s));
+  gp::UnsupportedInput in;
+  std::memset(&in, 0, sizeof in);
+  in.miss = ctx->d_sup_miss.as<uint32_t>();
+  in.draft_words = ctx->sup_draft_words;
+  in.polished_words = ctx->sup_polished_words;
+  in.draft_off = ctx->d_in_off.as<uint64_t>();
+  in.cap_off = ctx->d_cap_off.as<uint64_t>();
+  in.seg_off = ctx->d_uns_seg.as<uint64_t>();
+  in.n_seg = n_seg;
+  in.nk = nk;
+  for (uint32_t j = 0; j < nk; j++) in.k[j] = ctx->cfg.k[j];
+  uint64_t* run_cnt = ctx->d_uns_runcnt.as<uint64_t>();
+  uint32_t* miss_cnt = ctx->d_uns_misscnt.as<uint32_t>();
+  size_t tmp = 0;
+  GP_CUDA(ctx, gp::unsupported_count(in, n_words, run_cnt, miss_cnt, nullptr, tmp, s));
+  GP_CUDA(ctx, ctx->d_uns_tmp.ensure(std::max<size_t>(tmp, 16)));
+  tmp = ctx->d_uns_tmp.cap;
+  GP_CUDA(ctx, gp::unsupported_count(in, n_words, run_cnt, miss_cnt, ctx->d_uns_tmp.p, tmp, s));
+  uint64_t total = 0;
+  if (n_words) GP_CUDA(ctx, cudaMemcpyAsync(&total, run_cnt + n_words - 1, 8, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  GP_CUDA(ctx, ctx->d_uns_runs.ensure(std::max<uint64_t>(total, 1) * sizeof(gp_unsupported_run)));
+  if (total) GP_CUDA(ctx, cudaMemsetAsync(ctx->d_uns_runs.p, 0, total * sizeof(gp_unsupported_run), s));
+  GP_CUDA(ctx, gp::unsupported_fill(in, n_words, run_cnt, miss_cnt, ctx->d_uns_runs.as<gp_unsupported_run>(), ctx->d_uns_off.as<uint64_t>(), s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  ctx->n_unsupported = total;
+  ctx->unsupported_ready = true;
+  return GP_OK;
+}
+
+int gp_polish_fetch_unsupported(gp_ctx* ctx, uint64_t* run_off, gp_unsupported_run* runs, uint64_t cap, uint64_t* needed)
+{
+  if (!ctx || !run_off || !needed) return GP_ERR_ARG;
+  if (!ctx->cfg.kmer_support) GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch_unsupported needs gp_config.kmer_support = 1");
+  if (!ctx->polish_done || !ctx->support_polish)
+    GP_FAIL(ctx, GP_ERR_STATE, "gp_polish_fetch_unsupported before gp_polish_run / gp_pipeline_run");
+  cudaSetDevice(ctx->cfg.device);
+  cudaStream_t s = ctx->stream;
+  std::vector<uint32_t> len;
+  std::vector<uint8_t> dropped;
+  if (int rc = polish_settle(ctx, len, dropped)) return rc;
+  if (!ctx->unsupported_ready)
+    if (int rc = derive_unsupported(ctx, dropped)) return rc;
+  const size_t n_off = size_t(ctx->n_contigs) * 2 * ctx->cfg.nk + 1;
+  *needed = ctx->n_unsupported;
+  GP_CUDA(ctx, cudaMemcpyAsync(run_off, ctx->d_uns_off.p, n_off * 8, cudaMemcpyDeviceToHost, s));
+  GP_CUDA(ctx, cudaStreamSynchronize(s));
+  if (cap < ctx->n_unsupported || (ctx->n_unsupported && !runs))
+    GP_FAIL(ctx, GP_ERR_ARG, "run buffer too small (needed: *needed runs)");
+  if (ctx->n_unsupported) {
+    GP_CUDA(ctx, cudaMemcpyAsync(runs, ctx->d_uns_runs.p, ctx->n_unsupported * sizeof(gp_unsupported_run), cudaMemcpyDeviceToHost, s));
+    GP_CUDA(ctx, cudaStreamSynchronize(s));
+  }
   return GP_OK;
 }
 

@@ -175,8 +175,41 @@ struct SupportInput {
   uint32_t nk;
   uint32_t k[kMaxK];
 };
-// steps: 2 n words (record steps, scanned in place); tmp == nullptr: tmp_bytes receives the scan's scratch size
-cudaError_t support_count(const SupportInput& in, uint64_t* steps, void* tmp, size_t& tmp_bytes, int sm_count, cudaStream_t s);
+// Unsupported k-mer starts (valid and not contained), 1 bit per start position, addressed per contig: the part of record
+// r of contig c for k index j begins at word
+//   r = 0 (draft):    j * draft_words + draft_off[c] / 32 + c
+//   r = 1 (polished): nk * draft_words + j * polished_words + cap_off[c] / 32 + c
+// with draft_words = draft_off[n] / 32 + n and polished_words = cap_off[n] / 32 + n (room for ceil(len / 32) words each)
+struct SupportMiss {
+  uint32_t* bits;
+  uint64_t draft_words, polished_words;
+};
+// steps: 2 n words (record steps, scanned in place); tmp == nullptr: tmp_bytes receives the scan's scratch size.
+// Every step of every record of the launch also stores its 32 unsupported-start bits per k into miss.
+cudaError_t support_count(const SupportInput& in, const SupportMiss& miss, uint64_t* steps, void* tmp, size_t& tmp_bytes,
+                          int sm_count, cudaStream_t s);
+
+// Runs of unsupported k-mers (gp_polish_fetch_unsupported) from the bitmap of SupportMiss.  The words of every segment
+// (contig c, record r, k index j), segment (c * 2 + r) * nk + j, form one flat range: seg_off[s] .. seg_off[s + 1]
+// (ceil(len / 32) words of a record of len >= k, else none).
+struct UnsupportedInput {
+  const uint32_t* miss;
+  uint64_t draft_words, polished_words;
+  const uint64_t* draft_off;
+  const uint64_t* cap_off;
+  const uint64_t* seg_off;
+  uint32_t n_seg;
+  uint32_t nk;
+  uint32_t k[kMaxK];
+};
+// per word of the flat range: run starts into run_cnt and unsupported starts into miss_cnt, both scanned in place
+// (inclusive; miss_cnt wraps modulo 2^32, only differences inside a run are used).  tmp == nullptr: tmp_bytes receives
+// the scans' scratch size.
+cudaError_t unsupported_count(const UnsupportedInput& in, uint64_t n_words, uint64_t* run_cnt, uint32_t* miss_cnt, void* tmp,
+                              size_t& tmp_bytes, cudaStream_t s);
+// runs[] (zeroed by the caller) and run_off[0 .. n_seg] from the scanned counts
+cudaError_t unsupported_fill(const UnsupportedInput& in, uint64_t n_words, const uint64_t* run_scan, const uint32_t* miss_scan,
+                             gp_unsupported_run* runs, uint64_t* run_off, cudaStream_t s);
 // set bits of the nk filters of n_batches batches (batches[i], or first_batch + i without a list) into bits[batch * nk + ki]
 cudaError_t support_popcount(const uint32_t* bf_pool, const uint32_t* bf_slot, const uint32_t* batches, uint32_t first_batch,
                              uint32_t n_batches, uint32_t nk, unsigned long long* bits, cudaStream_t s);

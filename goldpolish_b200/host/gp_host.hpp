@@ -934,6 +934,47 @@ inline void write_kmer_qv(const std::string& path, const std::vector<std::string
 }
 
 // ---------------------------------------------------------------------------------------
+// runs of unsupported k-mers (gp_polish_fetch_unsupported) as BED rows
+// ---------------------------------------------------------------------------------------
+struct UnsupportedRuns {
+  std::vector<uint64_t> off;             // n_contigs * 2 * nk + 1: runs of (c, r, j) at off[(c * 2 + r) * nk + j] ..
+  std::vector<gp_unsupported_run> runs;
+};
+
+inline UnsupportedRuns fetch_unsupported(gp_ctx* ctx, uint32_t n_contigs, uint32_t nk)
+{
+  UnsupportedRuns u;
+  u.off.resize(size_t(n_contigs) * 2 * nk + 1);
+  uint64_t needed = 0;
+  int rc = gp_polish_fetch_unsupported(ctx, u.off.data(), nullptr, 0, &needed);
+  if (rc == GP_ERR_ARG && needed) {
+    u.runs.resize(needed);
+    rc = gp_polish_fetch_unsupported(ctx, u.off.data(), u.runs.data(), needed, &needed);
+  }
+  check_gp(ctx, rc, "gp_polish_fetch_unsupported");
+  return u;
+}
+
+// name<TAB>start<TAB>end<TAB>k<K><TAB>kmers for the runs of record r (0 draft, 1 polished) of every input record whose
+// emit[c] is set, by input record, then k in chain order, then start
+inline void write_unsupported_bed(const std::string& path, const std::vector<std::string>& names, const std::vector<uint32_t>& ks,
+                                  const UnsupportedRuns& u, uint32_t r, const std::vector<uint8_t>& emit)
+{
+  const size_t nk = ks.size();
+  std::ofstream o(path);
+  if (!o.good()) die("cannot write " + path);
+  for (size_t c = 0; c < names.size(); c++) {
+    if (!emit[c]) continue;
+    for (size_t j = 0; j < nk; j++) {
+      const size_t i = (c * 2 + r) * nk + j;
+      for (uint64_t x = u.off[i]; x < u.off[i + 1]; x++)
+        o << names[c] << '\t' << u.runs[x].start << '\t' << u.runs[x].end << "\tk" << ks[j] << '\t' << u.runs[x].kmers << '\n';
+    }
+  }
+  if (!o.good()) die("cannot write " + path);
+}
+
+// ---------------------------------------------------------------------------------------
 // FASTA/FASTQ reader with kseq semantics: gz or plain, multi-line sequences, name = text up
 // to the first whitespace, comment = rest of the header line
 // ---------------------------------------------------------------------------------------

@@ -5,7 +5,9 @@
 // intermediates of the script are not consumed by anything downstream.  GP_EDITS_VCF=1 also writes
 // <outfile>.edits.vcf: what the whole chain changed, in draft coordinates (header only when the guard keeps the input).
 // GP_KMER_QV=1 writes <outfile>.kmer_qv.tsv: k-mer completeness and QV of every record, draft and polished, for every k
-// of the chain (when the guard keeps the input, the polished columns describe it).
+// of the chain (when the guard keeps the input, the polished columns describe it).  GP_KMER_BED=1 writes
+// <outfile>.kmer_unsupported.bed: the runs of unsupported k-mers of what <outfile> holds, for every k of the chain (the
+// polished records, or the draft's runs when the guard keeps the input).
 #include "gp_host.hpp"
 
 #include <sys/stat.h>
@@ -50,7 +52,9 @@ int main(int argc, char** argv)
   const char* vcf_env = std::getenv("GP_EDITS_VCF");
   cfg.track_edits = vcf_env && std::string(vcf_env) == "1";
   const char* qv_env = std::getenv("GP_KMER_QV");
-  cfg.kmer_support = qv_env && std::string(qv_env) == "1";
+  const char* bed_env = std::getenv("GP_KMER_BED");
+  const bool kmer_qv = qv_env && std::string(qv_env) == "1", kmer_bed = bed_env && std::string(bed_env) == "1";
+  cfg.kmer_support = kmer_qv || kmer_bed;
   const std::string in_path = base + ".fa";
   struct stat st;
   if (stat(in_path.c_str(), &st) != 0) die("cannot stat " + in_path);
@@ -75,7 +79,9 @@ int main(int argc, char** argv)
   EditRecords er;
   if (cfg.track_edits) er = fetch_edits(ctx, uint32_t(recs.size()));
   KmerSupport ks;
-  if (cfg.kmer_support) ks = fetch_support(ctx, uint32_t(recs.size()), cfg.nk, 1);
+  if (kmer_qv) ks = fetch_support(ctx, uint32_t(recs.size()), cfg.nk, 1);
+  UnsupportedRuns ur;
+  if (kmer_bed) ur = fetch_unsupported(ctx, uint32_t(recs.size()), cfg.nk);
   gp_ctx_destroy(ctx);
   // the chain's last file, named as the script's loop names it (:27-28)
   std::string prev = base;
@@ -113,7 +119,15 @@ int main(int argc, char** argv)
     for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); lens.push_back(off[i + 1] - off[i]); }
     write_edits_vcf(outfile + ".edits.vcf", names, lens, gp_guard_rejects(input_size, output_size) ? nullptr : &er);
   }
-  if (cfg.kmer_support) {
+  if (kmer_bed) { // the runs of what <outfile> will hold: the polished records, or the input when the guard keeps it
+    const bool rejected = gp_guard_rejects(input_size, output_size) != 0;
+    std::vector<std::string> names;
+    std::vector<uint8_t> emit;
+    for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); emit.push_back(rejected || !dropped[i] ? 1 : 0); }
+    write_unsupported_bed(outfile + ".kmer_unsupported.bed", names, std::vector<uint32_t>(cfg.k, cfg.k + cfg.nk), ur,
+                          rejected ? 0 : 1, emit);
+  }
+  if (kmer_qv) {
     std::vector<std::string> names;
     for (const auto& r : recs) names.push_back(r.name);
     write_kmer_qv(outfile + ".kmer_qv.tsv", names, std::vector<uint32_t>(cfg.k, cfg.k + cfg.nk), ks,

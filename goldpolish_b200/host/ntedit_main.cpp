@@ -26,6 +26,7 @@ const struct option longopts[] = {                                   // :124-147
   { "bed", required_argument, nullptr, 3 }, // extension: write the flagged (soft-masked, -a1) regions as BED rows
   { "vcf", required_argument, nullptr, 4 }, // extension: write what polishing changed as VCF records (draft coordinates)
   { "kmer-qv", required_argument, nullptr, 5 }, // extension: write k-mer completeness / QV of the draft and the polished records
+  { "kmer-bed", required_argument, nullptr, 6 }, // extension: write the runs of unsupported k-mers of the polished records as BED
   { nullptr, 0, nullptr, 0 }
 };
 void assert_readable(const std::string& p)
@@ -43,7 +44,7 @@ int main(int argc, char** argv)
   gp_default_config(&cfg);
   cfg.max_insertions = 5; cfg.max_deletions = 5; cfg.mode = 0; cfg.mask = 0; // ntedit.cpp:86-87,109,111
   cfg.use_ratio = 0;
-  std::string draft, bloom, bloomrep, prefix, bed, vcf, kmer_qv;
+  std::string draft, bloom, bloomrep, prefix, bed, vcf, kmer_qv, kmer_bed;
   unsigned nthreads = 1;
   int snv = 0, verbose = 0;
   bool dieflag = false;
@@ -75,6 +76,7 @@ int main(int argc, char** argv)
     case 3: arg >> bed; break;
     case 4: arg >> vcf; break;
     case 5: arg >> kmer_qv; break;
+    case 6: arg >> kmer_bed; break;
     default: break;
     }
     if (optarg != nullptr && (!arg.eof() || arg.fail())) { // :1944-1947
@@ -114,7 +116,7 @@ int main(int argc, char** argv)
   }
   if (const char* d = std::getenv("GP_DEVICE")) cfg.device = std::atoi(d);
   cfg.track_edits = vcf.empty() ? 0 : 1;
-  cfg.kmer_support = kmer_qv.empty() ? 0 : 1;
+  cfg.kmer_support = kmer_qv.empty() && kmer_bed.empty() ? 0 : 1;
 
   const std::vector<FastaRecord> recs = read_fasta(draft);
   std::string all;
@@ -166,6 +168,12 @@ int main(int argc, char** argv)
     std::vector<std::string> names;
     for (const auto& r : recs) names.push_back(r.name);
     write_kmer_qv(kmer_qv, names, { cfg.k[0] }, fetch_support(ctx, uint32_t(recs.size()), 1, 1), false);
+  }
+  if (!kmer_bed.empty()) { // the emitted records, coordinates of the polished record
+    std::vector<std::string> names;
+    std::vector<uint8_t> emit;
+    for (size_t i = 0; i < recs.size(); i++) { names.push_back(recs[i].name); emit.push_back(dropped[i] ? 0 : 1); }
+    write_unsupported_bed(kmer_bed, names, { cfg.k[0] }, fetch_unsupported(ctx, uint32_t(recs.size()), 1), 1, emit);
   }
   gp_ctx_destroy(ctx);
   return 0;

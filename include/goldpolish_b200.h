@@ -31,6 +31,9 @@
  *   gp_polish_fetch_support  k-mer completeness of the draft and of the polished record against the batch's filters,
  *                        as Merqury reports it from a k-mer database of its own.  No reference counterpart; the counts
  *                        mirror btllib::NtHash iteration and KmerBloomFilter::contains
+ *   gp_polish_fetch_unsupported  where the reads do not support the draft and the polished record: runs of positions
+ *                        covered by k-mers the batch's filter does not contain, as Merqury's BED of them.  No reference
+ *                        counterpart; the same k-mers as gp_polish_fetch_support
  *   gp_kmer_threshold    mappings_bases_to_kmer_threshold, src/goldpolish_targeted_bfs.cpp:45-53
  *   gp_mappings_cap      mappings_num_max, src/goldpolish_targeted_bfs.cpp:96-99
  */
@@ -94,7 +97,8 @@ typedef struct {
    * the edits (default 0).  Not combinable with prep_mode 2: hard-masked bases would read as substitutions. */
   int32_t track_edits;
   /* 1: count, for every contig and k, how many k-mers of its draft and of its polished record the filters of its batch
-   * contain, so that gp_polish_fetch_support can report k-mer completeness / QV (default 0: no buffers, no launches) */
+   * contain, so that gp_polish_fetch_support can report k-mer completeness / QV, and keep where the missing ones lie,
+   * for gp_polish_fetch_unsupported (default 0: no buffers, no launches) */
   int32_t kmer_support;
 } gp_config;
 
@@ -261,6 +265,26 @@ typedef struct { uint64_t draft_kmers, draft_present, polished_kmers, polished_p
  * batch-major, the set bits of every filter the polish used.  The same numbers before or after gp_polish_fetch /
  * gp_polish_fetch_edits (like them it settles a polish that has to run again). */
 int gp_polish_fetch_support(gp_ctx* ctx, gp_kmer_support* out, uint64_t* filter_bits_set);
+
+/* Where the k-mers the support counts call missing lie.  For contig c, record R (the draft, or the polished record as
+ * gp_polish_fetch_support defines it) and k index j:
+ *   a k-mer start p is UNSUPPORTED when its k-mer is valid under the rule above (all k bases ACGTacgt) and the filter of
+ *                    batch contig_batch[c] for k_j does not contain it
+ *   an unsupported RUN is a maximal run of positions that lie in the span [p, p + k) of at least one unsupported k-mer:
+ *                    0-based, half-open, in R's coordinates; spans that overlap or touch form one run (as bedtools
+ *                    merge joins them).  Windows holding N or IUPAC bases are no k-mers, so a gap alone is never a run.
+ *   kmers            the number of unsupported k-mer starts inside the run.  A span never crosses a run boundary, so
+ *                    over the runs of (c, R, j) kmers sums to kmers - present of gp_polish_fetch_support.
+ * A dropped contig has no polished runs; its draft runs are still reported. */
+typedef struct { uint32_t start, end, kmers; } gp_unsupported_run;
+/* runs of the last gp_polish / gp_pipeline_run; needs cfg.kmer_support (else GP_ERR_STATE, as before a polish).
+ * run_off: n_contigs * 2 * nk + 1 entries; runs of (contig c, record r: 0 draft / 1 polished, k index j) are
+ * runs[run_off[(c*2 + r)*nk + j] .. +1), ascending start.  cap too small -> GP_ERR_ARG, *needed = total
+ * (run_off filled either way; runs may be NULL with cap 0).  Derived on the device at the first call after a polish
+ * (the filters may be gone by then: the pass keeps the positions of the unsupported k-mers); the same result before or
+ * after gp_polish_fetch, gp_polish_fetch_edits and gp_polish_fetch_support, and like them it settles a polish that has
+ * to run again. */
+int gp_polish_fetch_unsupported(gp_ctx* ctx, uint64_t* run_off, gp_unsupported_run* runs, uint64_t cap, uint64_t* needed);
 
 /* ---- flagged regions ---------------------------------------------------------------- */
 /* The reference flags what it could not fix by soft-masking: ntEdit -a1 lower-cases the draft base at every position
